@@ -111,6 +111,24 @@ def shard(total, n, r):
     return total * r // n, total * (r + 1) // n
 
 
+DUMP_MAX_ROWS = 1 << 20  # per array (8 MiB as float64): the six files a dump can hold stay under 64 MiB
+DUMP_SEED = 20261017
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float64 (every value here is an integer below 2**53, so exact).
+    An array longer than DUMP_MAX_ROWS is replaced by a fixed seeded sample of its rows, and the sampled row
+    numbers go to <name>_rows.npy: the same output always yields the same files."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, np.float64)
+        if len(a) > DUMP_MAX_ROWS:
+            rows = np.sort(np.random.default_rng(DUMP_SEED).choice(len(a), DUMP_MAX_ROWS, replace=False))
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def host_threads():
     """Host threads the CPU arm may use: the affinity mask, capped by the cgroup CPU quota if one is set (a
     GPU slice of a shared host often sees every core but may run only a share of them)."""
@@ -266,7 +284,14 @@ def main():
     ap.add_argument("--launch", default="auto", choices=["auto", "graph", "eager"],
                     help="auto: both ways are tried for a few steps after the warm-up and the faster one is timed; graph: each step (status sweep on its side stream + select + fused gather + peer wait) is captured once per "
                          "parity as a CUDA graph and replayed; eager: one C-ABI call per launch group")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's assignment vector, the sweep's changed "
+                         "slot list and codes) as DIR/<name>.npy, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "rpk":
+        ap.error("--dump-outputs writes what the GPU arm computed; the reference arm times a pod sample that varies from run to run")
     args.warmup = max(args.warmup, 3) if args.impl == "rpk" else args.warmup
 
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
@@ -386,6 +411,18 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    def changed_list(par):
+        """(slot ids, codes) of the sweep that last wrote result set `par`.  p2p: every rank's region of this rank's
+        exchange buffer, in rank order (global slot ids); otherwise this rank's own list (local slot ids)."""
+        if p2p:
+            xv = xchg_views[par].cpu().numpy()
+            counts = xv[:world].astype(np.int64)
+            idx = np.concatenate([xv[8 + r * cap: 8 + r * cap + counts[r]] for r in range(world)]).astype(np.uint32)
+            codes16 = xv[8 + world * cap:].view(np.uint16)
+            return idx, np.concatenate([codes16[r * cap: r * cap + counts[r]] for r in range(world)])
+        n = int(d_nchanged.item())
+        return d_changed[:n].cpu().numpy().astype(np.uint32), d_code[:n].cpu().numpy().view(np.uint16)
+
     sampler = ClockSampler(local_rank)  # clocks under this load: polled from the warm-up through the timed steps
     sampler.start()
     for i in range(args.warmup):
@@ -501,6 +538,9 @@ def main():
     wall = time.perf_counter() - wall0
     launches = (launches_per_step * args.steps) if graphs is not None else (eng.launch_count() - launches0)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:  # before the breakdown pass below runs more steps
+        idx, codes = changed_list(executed[-1])
+        dump_outputs(args.dump_outputs, {"best": best_sets[executed[-1]].cpu().numpy(), "status_changed": idx, "status_codes": codes})
     tot_ms = [e[0].elapsed_time(e[1]) for e in evs]        # whole step: select (+ gather) with the status sweep alongside
     if graphs is not None:
         # per-kernel breakdown: timing events cannot sit inside a captured graph, so the same steps run once more
@@ -546,18 +586,10 @@ def main():
         sel = check_select_parity(best_sets[last_par].cpu().numpy(), offers, pods_all, oracle, threads)
         tabs = recs_np if world == 1 else [synth.make_status_records(NS, 0), synth.make_status_records(NS, 1, 0.01)]
         prev_par = executed[-2] if len(executed) > 1 else last_par
-        if p2p:  # the gathered result: every rank's region of this rank's exchange buffer, in rank order
-            xv = xchg_views[last_par].cpu().numpy()
-            counts = xv[:world].astype(np.int64)
-            idx = np.concatenate([xv[8 + r * cap: 8 + r * cap + counts[r]] for r in range(world)]).astype(np.uint32)
-            codes16 = xv[8 + world * cap:].view(np.uint16)
-            codes = np.concatenate([codes16[r * cap: r * cap + counts[r]] for r in range(world)])
-            n_changed = int(counts.sum())
-        else:
-            idx = d_changed[:n_changed].cpu().numpy().astype(np.uint32)
-            codes = d_code[:n_changed].cpu().numpy().view(np.uint16)
-            if world > 1:  # NCCL comparison mode: each rank checks its own shard (local slot ids)
-                tabs = recs_np
+        idx, codes = changed_list(last_par)
+        n_changed = len(idx)
+        if world > 1 and not p2p:  # NCCL comparison mode: each rank checks its own shard (local slot ids)
+            tabs = recs_np
         st = check_status_parity(idx, codes, tabs[prev_par], tabs[last_par], oracle)
         flag = torch.tensor([int(sel["ok"] and st["ok"])], dtype=torch.int32, device=dev)
         if world > 1:
