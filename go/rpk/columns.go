@@ -48,3 +48,17 @@ func ReqMemColumn(v string) int32 {
 	}
 	return int32(mem)
 }
+
+// GpuTypeIDs parses runpod.io/gpu-type-ids exactly like runpod.io/datacenter-ids (runpod_client.go:1354-1362):
+// strings.Split on "," then strings.TrimSpace per element (empty elements are kept; they match no GPU type).
+// "" (annotation absent, after AnnotationWithFallback) = nil: the pod is not restricted.
+func GpuTypeIDs(v string) []string {
+	if v == "" {
+		return nil
+	}
+	ids := strings.Split(v, ",")
+	for i, id := range ids {
+		ids[i] = strings.TrimSpace(id)
+	}
+	return ids
+}

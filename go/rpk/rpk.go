@@ -154,6 +154,73 @@ func (e *Engine) Select(p *Pods, wantTop5 bool) (best []int32, top5 []int32, err
 	return best, top5, nil
 }
 
+// MaxOfferSets is the most offer sets one UploadOfferSets call holds; SetAll marks an unrestricted row.
+const (
+	MaxOfferSets        = C.RPK_MAX_OFFER_SETS
+	SetAll       uint16 = C.RPK_SET_ALL
+)
+
+func u16p(s []uint16) *C.uint16_t {
+	if len(s) == 0 {
+		return nil
+	}
+	return (*C.uint16_t)(unsafe.Pointer(&s[0]))
+}
+
+// UploadOfferSets replaces every offer set: set s holds the offer indices sets[s] of the resident table (indices
+// outside [0, G) are ignored).  A later UploadOffers makes the sets stale (SelectSets then fails until they are
+// uploaded again).  len(sets) = 0 clears them.
+func (e *Engine) UploadOfferSets(sets [][]int32) error {
+	e.mu.Lock()
+	defer e.mu.Unlock()
+	if len(sets) > MaxOfferSets {
+		return fmt.Errorf("rpk: %d offer sets, at most %d per upload", len(sets), MaxOfferSets)
+	}
+	w := (e.g + 31) / 32
+	words := make([]uint32, len(sets)*w)
+	for s, members := range sets {
+		for _, g := range members {
+			if g >= 0 && int(g) < e.g {
+				words[s*w+int(g)/32] |= 1 << (uint(g) & 31)
+			}
+		}
+	}
+	var wp *C.uint32_t
+	if len(words) > 0 {
+		wp = (*C.uint32_t)(unsafe.Pointer(&words[0]))
+	}
+	if rc := C.rpk_offer_sets_upload(e.ctx, C.uint32_t(len(sets)), C.uint32_t(e.g), wp); rc != C.RPK_OK {
+		return lastError(e.ctx, rc)
+	}
+	return nil
+}
+
+// SelectSets is Select with pod p restricted to offer set setID[p] (SetAll = the whole table; an id without a set
+// = nothing feasible): GetGPUTypes over the set's members only, indices into the whole table.
+func (e *Engine) SelectSets(p *Pods, setID []uint16, wantTop5 bool) (best []int32, top5 []int32, err error) {
+	e.mu.Lock()
+	defer e.mu.Unlock()
+	n := len(p.ReqMemGb)
+	best = make([]int32, n)
+	if n == 0 {
+		return best, nil, nil
+	}
+	if setID != nil && len(setID) != n {
+		return nil, nil, fmt.Errorf("rpk: %d set ids for %d pods", len(setID), n)
+	}
+	var t5 *C.int32_t
+	if wantTop5 {
+		top5 = make([]int32, n*TopK)
+		t5 = i32p(top5)
+	}
+	rc := C.rpk_select_sets(e.ctx, C.uint32_t(n), i32p(p.ReqMemGb), i32p(p.ReqVCPU), i32p(p.ReqRAMGb),
+		f64p(p.MaxPrice), u8p(p.Cloud), u16p(setID), i32p(best), t5)
+	if rc != C.RPK_OK {
+		return nil, nil, lastError(e.ctx, rc)
+	}
+	return best, top5, nil
+}
+
 // StatusDiff is the batched predicate of updateAllPodStatuses (kubelet.go:870-873): records holds one
 // fixed slot per tracked pod (see EncodeStatusRecord); the indices of the slots whose (status, ports)
 // pair differs from the previous sweep come back ascending.

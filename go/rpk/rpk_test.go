@@ -186,3 +186,85 @@ func TestStatusDiff(t *testing.T) {
 		t.Errorf("changed = %v, want %v", got, want)
 	}
 }
+
+// runpod.io/gpu-type-ids: parsed like runpod.io/datacenter-ids (runpod_client.go:1354-1362).
+func TestGpuTypeIDs(t *testing.T) {
+	cases := []struct {
+		in   string
+		want []string
+	}{
+		{"", nil},
+		{"A40", []string{"A40"}},
+		{" A40 , L4\t,A100 ", []string{"A40", "L4", "A100"}},
+		{"A40,,L4", []string{"A40", "", "L4"}},
+		{",", []string{"", ""}},
+	}
+	for _, c := range cases {
+		if got := GpuTypeIDs(c.in); !reflect.DeepEqual(got, c.want) {
+			t.Errorf("GpuTypeIDs(%q) = %q, want %q", c.in, got, c.want)
+		}
+	}
+}
+
+// The offer-set known answers of tests/golden/select_sets_kat.json: a restricted pod gets GetGPUTypes over its
+// set's members only, table indices out, ties to the lower table index whatever the list order.
+func TestSelectSetsKnownAnswers(t *testing.T) {
+	e, err := New(1)
+	if err != nil {
+		t.Skipf("no B200: %v", err)
+	}
+	defer e.Close()
+	if err := e.UploadOffers(katOffers()); err != nil {
+		t.Fatal(err)
+	}
+	sets := [][]int32{{1, 3, 5}, {2}, {4, 2, 1}, {6, 7, 9}, {}} // {A5000, A40, L4}, {RTX3090}, ..., ids not in the table
+	if err := e.UploadOfferSets(sets); err != nil {
+		t.Fatal(err)
+	}
+	cases := []struct {
+		name     string
+		minMem   int32
+		maxPrice float64
+		cloud    uint8
+		set      uint16
+		want     []int32
+	}{
+		{"price order inside the set", 16, 0.5, CloudSecure, 0, []int32{1, 3, 5}},
+		{"only member has no secure flag", 16, 0.5, CloudSecure, 1, []int32{}},
+		{"tie 0.22 -> lower table index", 24, 0.5, CloudCommunity, 2, []int32{1, 2, 4}},
+		{"price 0 excluded; 0.5 < 2.0", 16, 2.0, CloudSecure, 3, []int32{9, 6}},
+		{"empty set", 16, 0.5, CloudSecure, 4, []int32{}},
+		{"id without a set", 16, 0.5, CloudSecure, 17, []int32{}},
+		{"unrestricted = the reference KAT", 16, 0.5, CloudSecure, SetAll, []int32{0, 8, 1, 3, 5}},
+	}
+	batch := &Pods{}
+	var ids []uint16
+	for _, c := range cases {
+		batch.ReqMemGb = append(batch.ReqMemGb, c.minMem)
+		batch.MaxPrice = append(batch.MaxPrice, c.maxPrice)
+		batch.Cloud = append(batch.Cloud, c.cloud)
+		ids = append(ids, c.set)
+	}
+	best, top5, err := e.SelectSets(batch, ids, true)
+	if err != nil {
+		t.Fatal(err)
+	}
+	for i, c := range cases {
+		if got := trim(top5[i*TopK : (i+1)*TopK]); !reflect.DeepEqual(got, c.want) {
+			t.Errorf("%s: gpuTypeIds = %v, want %v", c.name, got, c.want)
+		}
+		wantBest := int32(-1)
+		if len(c.want) > 0 {
+			wantBest = c.want[0]
+		}
+		if best[i] != wantBest {
+			t.Errorf("%s: best = %d, want %d", c.name, best[i], wantBest)
+		}
+	}
+	if err := e.UploadOffers(katOffers()); err != nil { // a new table makes the sets stale
+		t.Fatal(err)
+	}
+	if _, _, err := e.SelectSets(batch, ids, false); err == nil {
+		t.Errorf("SelectSets after UploadOffers: want an error (stale offer sets)")
+	}
+}

@@ -14,6 +14,7 @@ package vk
 import (
 	"context"
 	"fmt"
+	"sort"
 	"strings"
 	"sync"
 	"time"
@@ -30,6 +31,9 @@ const (
 	CloudTypeAnnotation = "runpod.io/cloud-type"
 	GpuMemoryAnnotation = "runpod.io/required-gpu-memory"
 	PortsAnnotation     = "runpod.io/ports"
+
+	// extension of this build: the GPU types a pod may run on, comma-separated (parsed like runpod.io/datacenter-ids)
+	GpuTypeIdsAnnotation = "runpod.io/gpu-type-ids"
 )
 
 // InstanceInfo mirrors runpod_client.go:98-109 plus the slot of the device-resident previous-state column.
@@ -67,6 +71,10 @@ type Provider struct {
 	engine  *rpk.Engine
 	offers  *rpk.Offers
 	maxPods int
+
+	offerUploads int      // tables uploaded so far
+	setLists     []string // offer sets resident on the engine: set s = the canonical id list setLists[s]
+	setTable     int      // ... built on table upload number setTable
 
 	podsMutex sync.RWMutex // kubelet.go:38-45
 	pods      map[string]*v1.Pod
@@ -238,12 +246,14 @@ func (p *Provider) processPendingPods() {
 func (p *Provider) deployBatch(keys []string) {
 	cols := &rpk.Pods{}
 	var pods []*v1.Pod
+	var gpuTypes []string // raw runpod.io/gpu-type-ids per row, "" = unrestricted
 	p.podsMutex.RLock()
 	for _, k := range keys {
 		if pod, ok := p.pods[k]; ok {
 			job := p.api.OwnerJobAnnotations(pod)
 			cols.ReqMemGb = append(cols.ReqMemGb, rpk.ReqMemColumn(rpk.AnnotationWithFallback(pod.Annotations, job, GpuMemoryAnnotation, "")))
 			cols.Cloud = append(cols.Cloud, rpk.CloudColumn(rpk.AnnotationWithFallback(pod.Annotations, job, CloudTypeAnnotation, "")))
+			gpuTypes = append(gpuTypes, rpk.AnnotationWithFallback(pod.Annotations, job, GpuTypeIdsAnnotation, ""))
 			pods = append(pods, pod)
 		}
 	}
@@ -257,8 +267,18 @@ func (p *Provider) deployBatch(keys []string) {
 			return
 		}
 		p.offers = offers
+		p.offerUploads++
 	}
-	_, top5, err := p.engine.Select(cols, true)
+	restricted := false
+	for _, v := range gpuTypes {
+		restricted = restricted || v != ""
+	}
+	var top5 []int32
+	if !restricted { // no pod carries runpod.io/gpu-type-ids: the plain selection, exactly as without the annotation
+		_, top5, err = p.engine.Select(cols, true)
+	} else {
+		top5, err = p.selectWithSets(cols, gpuTypes)
+	}
 	if err != nil {
 		return
 	}
@@ -290,6 +310,128 @@ func (p *Provider) deployBatch(keys []string) {
 		}
 		p.podsMutex.Unlock()
 	}
+}
+
+// selectWithSets: every distinct gpu-type-ids list of the batch, as a set of ids, becomes an offer set (ids absent
+// from the table are ignored: a list that matches nothing gives an empty gpuTypeIds and the pod stays pending).  The
+// resident sets are reused while the table is unchanged and hold every list; otherwise the lists are uploaded,
+// rpk.MaxOfferSets at a time, each group with one SelectSets over its rows (unrestricted rows go with the first group).
+// A failed reuse (sets gone stale on the engine) falls back to uploading once.
+func (p *Provider) selectWithSets(cols *rpk.Pods, gpuTypes []string) ([]int32, error) {
+	top5, err := p.selectWithSetsOnce(cols, gpuTypes, true)
+	if err != nil && p.setLists == nil {
+		top5, err = p.selectWithSetsOnce(cols, gpuTypes, false)
+	}
+	return top5, err
+}
+
+func (p *Provider) selectWithSetsOnce(cols *rpk.Pods, gpuTypes []string, mayReuse bool) ([]int32, error) {
+	n := len(gpuTypes)
+	listOf := map[string]int{}
+	var lists []string // canonical form: sorted unique ids joined by ","
+	rowList := make([]int, n)
+	for i, v := range gpuTypes {
+		rowList[i] = -1
+		if v == "" {
+			continue
+		}
+		ids := rpk.GpuTypeIDs(v)
+		sort.Strings(ids)
+		uniq := ids[:0]
+		for j, id := range ids {
+			if j == 0 || id != ids[j-1] {
+				uniq = append(uniq, id)
+			}
+		}
+		k := strings.Join(uniq, "\x00")
+		l, ok := listOf[k]
+		if !ok {
+			l = len(lists)
+			listOf[k] = l
+			lists = append(lists, k)
+		}
+		rowList[i] = l
+	}
+	indexOf := map[string]int32{}
+	for g, id := range p.offers.IDs {
+		if _, dup := indexOf[id]; !dup {
+			indexOf[id] = int32(g)
+		}
+	}
+	resident := make([]int, len(lists))
+	reuse := mayReuse && p.setLists != nil && p.setTable == p.offerUploads
+	for l := 0; reuse && l < len(lists); l++ {
+		resident[l] = -1
+		for s, k := range p.setLists {
+			if k == lists[l] {
+				resident[l] = s
+				break
+			}
+		}
+		reuse = resident[l] >= 0
+	}
+	groups := 1
+	if !reuse {
+		groups = (len(lists) + rpk.MaxOfferSets - 1) / rpk.MaxOfferSets
+	}
+	top5 := make([]int32, n*rpk.TopK)
+	for grp := 0; grp < groups; grp++ {
+		l0, l1 := grp*rpk.MaxOfferSets, (grp+1)*rpk.MaxOfferSets
+		if l1 > len(lists) {
+			l1 = len(lists)
+		}
+		if !reuse {
+			p.setLists = nil // nothing is resident until the upload succeeds
+			sets := make([][]int32, 0, l1-l0)
+			for _, k := range lists[l0:l1] {
+				var members []int32
+				for _, id := range strings.Split(k, "\x00") {
+					if g, ok := indexOf[id]; ok {
+						members = append(members, g)
+					}
+				}
+				sets = append(sets, members)
+			}
+			if err := p.engine.UploadOfferSets(sets); err != nil {
+				return nil, err
+			}
+			p.setLists, p.setTable = append([]string(nil), lists[l0:l1]...), p.offerUploads
+		}
+		var rows []int
+		for i, l := range rowList {
+			if (l < 0 && grp == 0) || (l >= l0 && l < l1) {
+				rows = append(rows, i)
+			}
+		}
+		if len(rows) == 0 {
+			continue
+		}
+		sub := &rpk.Pods{}
+		setID := make([]uint16, len(rows))
+		for j, i := range rows {
+			sub.ReqMemGb = append(sub.ReqMemGb, cols.ReqMemGb[i])
+			sub.Cloud = append(sub.Cloud, cols.Cloud[i])
+			switch {
+			case rowList[i] < 0:
+				setID[j] = rpk.SetAll
+			case reuse:
+				setID[j] = uint16(resident[rowList[i]])
+			default:
+				setID[j] = uint16(rowList[i] - l0)
+			}
+		}
+		_, t5, err := p.engine.SelectSets(sub, setID, true)
+		if err != nil {
+			if reuse {
+				p.setLists = nil // stale on the engine: the caller uploads once more
+			}
+			return nil, err
+		}
+		for j, i := range rows {
+			copy(top5[i*rpk.TopK:(i+1)*rpk.TopK], t5[j*rpk.TopK:(j+1)*rpk.TopK])
+		}
+	}
+	return top5, nil
 }
 
 // updateAllPodStatuses -- kubelet.go:816-974, batched; see the C++ mirror for the concurrency argument.

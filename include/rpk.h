@@ -62,8 +62,8 @@ extern "C" {
 typedef struct rpk_ctx rpk_ctx;
 
 typedef struct rpk_stats {
-    uint64_t select_calls;        /* rpk_select + rpk_select_device */
-    uint64_t offer_scores;        /* sum of P*G over those calls */
+    uint64_t select_calls;        /* rpk_select + rpk_select_device (+ the _sets variants) */
+    uint64_t offer_scores;        /* sum of P*G over those calls (sets: sum of P_s*G_s, the grid evaluated) */
     uint64_t status_calls;
     uint64_t status_records;      /* sum of N */
     float last_select_kernel_ms;  /* 0: rpk_select overlaps copies and kernels (sub-batch pipeline), only the total is meaningful */
@@ -179,6 +179,34 @@ int rpk_peer_wait(rpk_ctx* ctx, int shard, unsigned what, void* stream);
  * drives SEVERAL shards of a group must enable it only after one call of each size has sized the scratch: a call that
  * allocates synchronises its device, which would wait for a kernel that waits for a peer not launched yet. */
 int rpk_peer_inline_wait(rpk_ctx* ctx, int shard, int on);
+
+/* ---- offer sets: restrict a pod to a list of offers (runpod.io/gpu-type-ids) ------------------------ */
+
+/* An offer set is a sub-table: a pod restricted to set s gets exactly what rpk_select would give it against a table
+ * holding only the members of s, in their relative order -- same filter, same price order with ties to the lowest
+ * GLOBAL offer index, same <= 5 list -- and the indices returned are global offer indices. */
+#define RPK_MAX_OFFER_SETS 256
+#define RPK_SET_ALL 0xFFFFu   /* set_id value: unrestricted (the whole table, = rpk_select) */
+
+/* Set s = offers g of the resident table with bit (g & 31) of members[s*W + g/32] set, W = ceil(G/32); bits >= G are
+ * ignored.  G must equal the resident table's G (RPK_EINVAL otherwise).  Replaces all previous sets; n_sets = 0 clears
+ * them.  Built on every GPU of the ctx.  A later rpk_offers_upload makes the sets stale: rpk_select_sets then fails with
+ * RPK_ESTATE until the sets are uploaded again (indices would otherwise refer to another table). */
+int rpk_offer_sets_upload(rpk_ctx* ctx, uint32_t n_sets, uint32_t G, const uint32_t* members);
+
+/* rpk_select with one more column: set_id[p] restricts pod p to set set_id[p].  RPK_SET_ALL = the whole table;
+ * any other id >= n_sets behaves like an empty set (best -1, top5 all -1), the same convention as an unknown cloud byte.
+ * NULL set_id = every row RPK_SET_ALL = rpk_select's result (no sets need to be uploaded for that).  Does not write the
+ * device-resident full vector (rpk_best_device_ptr keeps the last rpk_select's). */
+int rpk_select_sets(rpk_ctx* ctx, uint32_t P, const int32_t* req_mem_gb, const int32_t* req_vcpu, const int32_t* req_ram_gb,
+                    const double* max_price, const uint8_t* cloud, const uint16_t* set_id, int32_t* best, int32_t* top5);
+/* Device-resident variant on GPU `shard`.  It reads back the per-set row counts once, so it synchronises `stream` once
+ * and cannot be captured in a CUDA graph: on a capturing stream it returns RPK_ESTATE before enqueuing anything (with
+ * d_set_id NULL it only enqueues, like rpk_select_device, and may be captured).  Shares the
+ * shard's select scratch with rpk_select_device (see rpk_status_diff_device). */
+int rpk_select_sets_device(rpk_ctx* ctx, int shard, uint32_t P, const int32_t* d_req_mem_gb, const int32_t* d_req_vcpu,
+                           const int32_t* d_req_ram_gb, const double* d_max_price, const uint8_t* d_cloud,
+                           const uint16_t* d_set_id, int32_t* d_best, int32_t* d_top5, void* stream);
 
 /* Device pointer of GPU `shard`'s copy of the full assignment vector written by the last rpk_select
  * (ctx-owned; every GPU of the ctx holds the whole vector after the call). */

@@ -22,7 +22,11 @@ SYMBOLS = [
     "rpk_launch_count", "rpk_ipc_alloc", "rpk_ipc_open", "rpk_ipc_close", "rpk_ipc_free", "rpk_peer_fence",
     "rpk_peer_bind", "rpk_peer_wait", "rpk_peer_inline_wait", "rpk_status_diff_codes", "rpk_status_seed_slots", "rpk_tick",
     "rpk_status_diff_device_codes", "rpk_xchg_bytes", "rpk_status_diff_device_gather",
+    "rpk_offer_sets_upload", "rpk_select_sets", "rpk_select_sets_device",
 ]
+
+RPK_MAX_OFFER_SETS = 256
+RPK_SET_ALL = 0xFFFF
 
 
 class RpkStats(C.Structure):
@@ -75,6 +79,12 @@ def load():
     L.rpk_select_device_gather.restype = C.c_int
     L.rpk_select_device_gather.argtypes = [vp, C.c_int, u32, i32p, i32p, i32p, f64p, u8p, C.c_int, C.POINTER(vp), u32,
                                            i32p, vp]
+    L.rpk_offer_sets_upload.restype = C.c_int
+    L.rpk_offer_sets_upload.argtypes = [vp, u32, u32, u32p]
+    L.rpk_select_sets.restype = C.c_int
+    L.rpk_select_sets.argtypes = [vp, u32, i32p, i32p, i32p, f64p, u8p, vp, i32p, i32p]
+    L.rpk_select_sets_device.restype = C.c_int
+    L.rpk_select_sets_device.argtypes = [vp, C.c_int, u32, i32p, i32p, i32p, f64p, u8p, vp, i32p, i32p, vp]
     L.rpk_best_device_ptr.restype = vp
     L.rpk_best_device_ptr.argtypes = [vp, C.c_int]
     L.rpk_status_diff.restype = C.c_int

@@ -204,7 +204,7 @@ __global__ void __launch_bounds__(256) k_offer_bitmap(BitmapArgs a) {
 
 static uint32_t bitlen(uint32_t x) { uint32_t b = 0; while (x) { ++b; x >>= 1; } return b ? b : 1; }
 
-int launch_offer_ingest(DeviceState& ds, const OfferIngest& in, cudaStream_t st) {
+int launch_offer_ingest(DeviceState& ds, OfferTable& t, const OfferIngest& in, cudaStream_t st) {
     int launches = 0;
     const uint32_t G = in.G;
     uint32_t n = 1024;
@@ -214,11 +214,11 @@ int launch_offer_ingest(DeviceState& ds, const OfferIngest& in, cudaStream_t st)
     ds.sort_keys.reserve((size_t)3 * n);
     ds.sort_vals.reserve((size_t)3 * n);
     for (int c = 0; c < 2; ++c) {
-        ds.v_bitmap[c].reserve((size_t)(Gpad / 32) * kBmMaxStride);
-        ds.v_bitmapT[c].reserve((size_t)(((G + 31) / 32 + kSubChunks - 1) / kSubChunks + 1) * kBmMaxStride * kSubStride);
-        ds.v_packed[c].reserve(Gpad); ds.v_wide[c].reserve(Gpad); ds.v_price[c].reserve(Gpad); ds.v_perm[c].reserve(Gpad);
+        t.v_bitmap[c].reserve((size_t)(Gpad / 32) * kBmMaxStride);
+        t.v_bitmapT[c].reserve((size_t)(((G + 31) / 32 + kSubChunks - 1) / kSubChunks + 1) * kBmMaxStride * kSubStride);
+        t.v_packed[c].reserve(Gpad); t.v_wide[c].reserve(Gpad); t.v_price[c].reserve(Gpad); t.v_perm[c].reserve(Gpad);
     }
-    for (int d = 0; d < 3; ++d) ds.distinct[d].reserve(G ? G : 1);
+    for (int d = 0; d < 3; ++d) t.distinct[d].reserve(G ? G : 1);
     ds.dcount.reserve(4);
     u64* keys = ds.sort_keys.p;
     uint32_t* vals = ds.sort_vals.p;
@@ -230,7 +230,7 @@ int launch_offer_ingest(DeviceState& ds, const OfferIngest& in, cudaStream_t st)
     for (int d = 0; d < 3; ++d) {
         k_dim_keys<<<(n + 255) / 256, 256, 0, st>>>(G, n, cols[d], keys + 2 * (size_t)n, vals + 2 * (size_t)n); ++launches;
         launches += bitonic_sort(keys + 2 * (size_t)n, vals + 2 * (size_t)n, n, st);
-        k_unique<<<1, 1024, 0, st>>>(keys + 2 * (size_t)n, G, ds.distinct[d].p, ds.dcount.p + d); ++launches;
+        k_unique<<<1, 1024, 0, st>>>(keys + 2 * (size_t)n, G, t.distinct[d].p, ds.dcount.p + d); ++launches;
     }
     uint32_t D[3] = {0, 0, 0};
     RPK_CUDA(cudaMemcpyAsync(D, ds.dcount.p, sizeof(D), cudaMemcpyDeviceToHost, st));
@@ -260,32 +260,122 @@ int launch_offer_ingest(DeviceState& ds, const OfferIngest& in, cudaStream_t st)
         pk.sh_ram = 0; pk.sh_vcpu = b3 + 1; pk.sh_mem = pk.sh_vcpu + b2 + 1;
         pk.guard = (1u << b3) | (1u << (pk.sh_vcpu + b2)) | (1u << (pk.sh_mem + b1));
     }
-    ds.nsub = 0;
+    t.nsub = 0;
     if (pk.bm_words) {
         BitmapArgs ba;
         ba.G = G; ba.nchunks = Gpad / 32; ba.keys = keys; ba.vals = vals; ba.n = n;
         ba.mem = in.mem; ba.vcpu = in.vcpu; ba.ram = in.ram;
-        for (int d = 0; d < 3; ++d) { ba.distinct[d] = ds.distinct[d].p; ba.D[d] = D[d]; }
+        for (int d = 0; d < 3; ++d) { ba.distinct[d] = t.distinct[d].p; ba.D[d] = D[d]; }
         ba.off_vcpu = pk.bm_off_vcpu; ba.off_ram = pk.bm_off_ram; ba.words = pk.bm_words; ba.stride = pk.bm_stride;
         ba.nchunks_real = (G + 31) / 32;
-        ds.nsub = (ba.nchunks_real + kSubChunks - 1) / kSubChunks;
+        t.nsub = (ba.nchunks_real + kSubChunks - 1) / kSubChunks;
         for (int c = 0; c < 2; ++c) {
-            ba.bitmap[c] = ds.v_bitmap[c].p; ba.bitmapT[c] = ds.v_bitmapT[c].p;
-            RPK_CUDA(cudaMemsetAsync(ds.v_bitmapT[c].p, 0, (size_t)(ds.nsub ? ds.nsub : 1) * pk.bm_words * kSubStride * sizeof(uint32_t), st));
+            ba.bitmap[c] = t.v_bitmap[c].p; ba.bitmapT[c] = t.v_bitmapT[c].p;
+            RPK_CUDA(cudaMemsetAsync(t.v_bitmapT[c].p, 0, (size_t)(t.nsub ? t.nsub : 1) * pk.bm_words * kSubStride * sizeof(uint32_t), st));
         }
         k_offer_bitmap<<<dim3((ba.nchunks * 32 + 255) / 256, 2), 256, 0, st>>>(ba); ++launches;
     }
     PackArgs pa;
     pa.G = G; pa.Gpad = Gpad; pa.n = n; pa.keys = keys; pa.vals = vals;
     pa.mem = in.mem; pa.vcpu = in.vcpu; pa.ram = in.ram; pa.sp = in.secure_price; pa.cp = in.community_price;
-    for (int d = 0; d < 3; ++d) { pa.distinct[d] = ds.distinct[d].p; pa.D[d] = D[d]; }
+    for (int d = 0; d < 3; ++d) { pa.distinct[d] = t.distinct[d].p; pa.D[d] = D[d]; }
     pa.pk = pk;
-    for (int c = 0; c < 2; ++c) { pa.packed[c] = ds.v_packed[c].p; pa.wide[c] = ds.v_wide[c].p; pa.price[c] = ds.v_price[c].p; pa.perm[c] = ds.v_perm[c].p; }
+    for (int c = 0; c < 2; ++c) { pa.packed[c] = t.v_packed[c].p; pa.wide[c] = t.v_wide[c].p; pa.price[c] = t.v_price[c].p; pa.perm[c] = t.v_perm[c].p; }
     k_offer_pack<<<dim3((Gpad + 255) / 256, 2), 256, 0, st>>>(pa); ++launches;
     RPK_CUDA(cudaGetLastError());
-    ds.G = G; ds.Gpad = Gpad; ds.pk = pk;
-    for (int d = 0; d < 3; ++d) ds.D[d] = D[d];
-    ds.offers_ready = true;
+    t.G = G; t.Gpad = Gpad; t.pk = pk;
+    for (int d = 0; d < 3; ++d) t.D[d] = D[d];
+    return launches;
+}
+
+// ---- offer sets ------------------------------------------------------------------------------------------
+// A set is a sub-table: its members, gathered in ascending global order, go through the same ingest as the resident
+// table.  Within the sub-table the (price, row) order is then the global (price, offer index) order, so the tie
+// contract holds, and one remap of perm / wide.w to global ids lets every select kernel emit global indices.
+
+// one block per set: popcount of each membership word, block-wide exclusive scan, each word's set bits written in
+// ascending order from its offset (bits >= G are ignored)
+__global__ void __launch_bounds__(1024) k_set_compact(const uint32_t* __restrict__ words, uint32_t W, uint32_t G,
+                                                      const uint32_t* __restrict__ set_off, uint32_t* __restrict__ members) {
+    __shared__ uint32_t warp_sum[32];
+    __shared__ uint32_t carry;
+    const uint32_t s = blockIdx.x, t = threadIdx.x, lane = t & 31, w = t >> 5;
+    const uint32_t* sw = words + (size_t)s * W;
+    uint32_t* out = members + set_off[s];
+    if (t == 0) carry = 0;
+    __syncthreads();
+    for (uint32_t base = 0; base < W; base += 1024) {
+        const uint32_t i = base + t;
+        uint32_t m = i < W ? sw[i] : 0u;
+        if (i < W && (i + 1) * 32 > G) m &= (1u << (G - i * 32)) - 1u;  // last word: 0 < G - 32 i < 32
+        const uint32_t c = __popc(m);
+        uint32_t incl = c;  // warp-inclusive scan of the counts
+        for (int d = 1; d < 32; d <<= 1) { const uint32_t v = __shfl_up_sync(0xFFFFFFFFu, incl, d); if (lane >= (uint32_t)d) incl += v; }
+        if (lane == 31) warp_sum[w] = incl;
+        __syncthreads();
+        uint32_t off = 0, total = 0;
+        for (uint32_t x = 0; x < 32; ++x) { const uint32_t v = warp_sum[x]; if (x < w) off += v; total += v; }
+        uint32_t pos = carry + off + incl - c;
+        while (m) { out[pos++] = i * 32 + (uint32_t)(__ffs(m) - 1); m &= m - 1; }
+        __syncthreads();
+        if (t == 0) carry += total;
+        __syncthreads();
+    }
+}
+
+// the six raw columns of the members (sub-table row j = offer members[j])
+__global__ void k_set_gather(uint32_t n, const uint32_t* __restrict__ members, const int32_t* __restrict__ mem,
+                             const int32_t* __restrict__ vcpu, const int32_t* __restrict__ ram, const double* __restrict__ sp,
+                             const double* __restrict__ cp, const uint8_t* __restrict__ flags, int32_t* __restrict__ o_mem,
+                             int32_t* __restrict__ o_vcpu, int32_t* __restrict__ o_ram, double* __restrict__ o_sp,
+                             double* __restrict__ o_cp, uint8_t* __restrict__ o_flags) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const uint32_t g = members[j];
+    o_mem[j] = mem[g]; o_vcpu[j] = vcpu[g]; o_ram[j] = ram[g]; o_sp[j] = sp[g]; o_cp[j] = cp[g]; o_flags[j] = flags[g];
+}
+
+// sub-table row -> global offer id in both views (-1 = unavailable / padding stays -1)
+__global__ void k_set_remap(uint32_t Gpad, const uint32_t* __restrict__ members, int32_t* perm0, int32_t* perm1, int4* wide0,
+                            int4* wide1) {
+    const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= Gpad) return;
+    int32_t* perm = blockIdx.y ? perm1 : perm0;
+    int4* wide = blockIdx.y ? wide1 : wide0;
+    const int32_t p = perm[s];
+    if (p >= 0) perm[s] = (int32_t)members[p];
+    const int32_t w = wide[s].w;
+    if (w >= 0) wide[s].w = (int32_t)members[w];
+}
+
+int launch_offer_sets_build(DeviceState& ds, uint32_t n_sets, const uint32_t* d_words, const uint32_t* counts, cudaStream_t st) {
+    int launches = 0;
+    const uint32_t G = ds.main.G, W = (G + 31) / 32;
+    std::vector<uint32_t> off((size_t)n_sets + 1, 0);
+    uint32_t gmax = 0;
+    for (uint32_t s = 0; s < n_sets; ++s) { off[s + 1] = off[s] + counts[s]; gmax = counts[s] > gmax ? counts[s] : gmax; }
+    ds.set_members.reserve((size_t)off[n_sets] + n_sets + 1);  // member lists, then the n_sets offsets
+    uint32_t* d_off = ds.set_members.p + off[n_sets];
+    RPK_CUDA(cudaMemcpyAsync(d_off, off.data(), (size_t)n_sets * 4, cudaMemcpyHostToDevice, st));
+    if (n_sets && W) { k_set_compact<<<n_sets, 1024, 0, st>>>(d_words, W, G, d_off, ds.set_members.p); ++launches; }
+    const size_t cap = gmax ? gmax : 1;
+    ds.set_mem.reserve(cap); ds.set_vcpu.reserve(cap); ds.set_ram.reserve(cap);
+    ds.set_sp.reserve(cap); ds.set_cp.reserve(cap); ds.set_flags.reserve(cap);
+    for (uint32_t s = 0; s < n_sets; ++s) {
+        OfferTable& t = ds.sets[s];
+        const uint32_t n = counts[s];
+        if (n == 0) { t.G = 0; continue; }  // an empty set never reaches a select kernel
+        const uint32_t* mem = ds.set_members.p + off[s];
+        k_set_gather<<<(n + 255) / 256, 256, 0, st>>>(n, mem, ds.raw_mem.p, ds.raw_vcpu.p, ds.raw_ram.p, ds.raw_sp.p, ds.raw_cp.p,
+                                                      ds.raw_flags.p, ds.set_mem.p, ds.set_vcpu.p, ds.set_ram.p, ds.set_sp.p,
+                                                      ds.set_cp.p, ds.set_flags.p);
+        ++launches;
+        OfferIngest in{n, ds.set_mem.p, ds.set_vcpu.p, ds.set_ram.p, ds.set_sp.p, ds.set_cp.p, ds.set_flags.p};
+        launches += launch_offer_ingest(ds, t, in, st);  // synchronises st once (distinct-value counts)
+        k_set_remap<<<dim3((t.Gpad + 255) / 256, 2), 256, 0, st>>>(t.Gpad, mem, t.v_perm[0].p, t.v_perm[1].p, t.v_wide[0].p, t.v_wide[1].p);
+        ++launches;
+    }
+    RPK_CUDA(cudaGetLastError());
     return launches;
 }
 

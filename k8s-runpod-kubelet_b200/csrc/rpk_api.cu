@@ -115,19 +115,19 @@ inline void shard_range(uint32_t total, int n, int s, uint32_t* lo, uint32_t* hi
     *hi = (uint32_t)((uint64_t)total * (uint64_t)(s + 1) / (uint64_t)n);
 }
 
-void fill_offer_args(const DeviceState& ds, SelectArgs& a) {
+void fill_offer_args(const OfferTable& t, SelectArgs& a) {
     for (int c = 0; c < 2; ++c) {
-        a.view[c].packed = ds.v_packed[c].p; a.view[c].bitmap = ds.v_bitmap[c].p; a.view[c].bitmapT = ds.v_bitmapT[c].p; a.view[c].wide = ds.v_wide[c].p;
-        a.view[c].price = ds.v_price[c].p; a.view[c].perm = ds.v_perm[c].p;
+        a.view[c].packed = t.v_packed[c].p; a.view[c].bitmap = t.v_bitmap[c].p; a.view[c].bitmapT = t.v_bitmapT[c].p; a.view[c].wide = t.v_wide[c].p;
+        a.view[c].price = t.v_price[c].p; a.view[c].perm = t.v_perm[c].p;
     }
-    a.G = ds.G; a.Gpad = ds.Gpad; a.pk = ds.pk; a.nsub = ds.nsub;
-    for (int d = 0; d < 3; ++d) { a.distinct[d] = ds.distinct[d].p; a.D[d] = ds.D[d]; }
+    a.G = t.G; a.Gpad = t.Gpad; a.pk = t.pk; a.nsub = t.nsub;
+    for (int d = 0; d < 3; ++d) { a.distinct[d] = t.distinct[d].p; a.D[d] = t.D[d]; }
 }
 
-// scratch for one select over P rows on ds (in lane ln); returns rows-per-warp.  *use_persist: the batch takes the
-// persistent bit-sliced kernel (plan in *pl).
-int prepare_select_scratch(DeviceState& ds, DeviceState::Lane& ln, uint32_t P, SelectArgs& a, PersistPlan* pl, bool* use_persist) {
-    const int R = ds.pk.bm_words ? 32 * pick_rows_per_lane(P, ds.G, ds.sm_count) : pick_rows_per_warp(P, ds.sm_count);
+// scratch for one select over P rows against table t of ds (in lane ln); returns rows-per-warp.  *use_persist: the batch
+// takes the persistent bit-sliced kernel (plan in *pl).
+int prepare_select_scratch(DeviceState& ds, const OfferTable& t, DeviceState::Lane& ln, uint32_t P, SelectArgs& a, PersistPlan* pl, bool* use_persist) {
+    const int R = t.pk.bm_words ? 32 * pick_rows_per_lane(P, t.G, ds.sm_count) : pick_rows_per_warp(P, ds.sm_count);
     const uint32_t tiles = select_tiles_max(P, R);
     ln.rw.reserve(P); ln.order.reserve((size_t)kGroups * P); ln.pos.reserve(P);
     const size_t need = std::max<size_t>((size_t)2 * kGroups + tiles, (size_t)P / 8 + 3 * kGroups);  // worst case (1 row per warp): never regrown mid-pipeline
@@ -141,10 +141,10 @@ int prepare_select_scratch(DeviceState& ds, DeviceState::Lane& ln, uint32_t P, S
     a.rw = ln.rw.p; a.order = ln.order.p; a.pos = ln.pos.p;
     a.counts = ln.ctrs.p; a.done = ln.ctrs.p + kGroups; a.tile_ctr = ln.ctrs.p + 2 * kGroups;
     a.P = P;
-    *use_persist = ds.pk.bm_words && (P > kFusedRowsMax || ds.pk.no_fused) && !ds.pk.no_persist && persist_plan(a, ds.sm_count, pl);
+    *use_persist = t.pk.bm_words && (P > kFusedRowsMax || t.pk.no_fused) && !t.pk.no_persist && persist_plan(a, ds.sm_count, pl);
     if (*use_persist) {
         ln.key.reserve(P); ln.ord_rw.reserve(P);
-        const size_t hdr_words = persist_hdr_words(ds.G, ds.pk.bm_words);
+        const size_t hdr_words = persist_hdr_words(t.G, t.pk.bm_words);
         const bool fresh = !ln.hist.p || hdr_words > ln.hdr.cap;
         ln.hist.reserve(2 * kMaxClasses); ln.cursor.reserve(2 * kMaxClasses); ln.hdr.reserve(hdr_words);
         if (fresh || ln.persist_dirty) {  // zero between calls by construction (k_pod_classify's last block, the pushers)
@@ -257,9 +257,9 @@ int select_small(rpk_ctx* ctx, DeviceState& ds, uint32_t P, const int32_t* req_m
     a.req_ram = req_ram_gb ? (const int32_t*)(d + o_ram) : nullptr; a.max_price = max_price ? (const double*)(d + o_price) : nullptr;
     a.cloud = cloud ? (const uint8_t*)(d + o_cloud) : nullptr;
     a.P = P;
-    fill_offer_args(ds, a);
+    fill_offer_args(ds.main, a);
     PersistPlan pl; bool persist = false;
-    const int R = prepare_select_scratch(ds, ln, P, a, &pl, &persist);
+    const int R = prepare_select_scratch(ds, ds.main, ln, P, a, &pl, &persist);
     a.best_out[0] = ds.d_small_out.p; a.n_out = 1; a.self_out = 0; a.row0 = 0; a.top5 = top5 ? ds.d_small_out.p + P : nullptr;
     *launches += (uint64_t)run_select(ln, a, R, persist ? &pl : nullptr, st);
     int32_t* hout = (int32_t*)(ds.h_small + in_cap);
@@ -333,9 +333,9 @@ void enqueue_select_shard(rpk_ctx* ctx, int s, uint32_t P, const int32_t* req_me
         a.req_mem = ln.p_req_mem.p; a.req_vcpu = req_vcpu ? ln.p_req_vcpu.p : nullptr; a.req_ram = req_ram_gb ? ln.p_req_ram.p : nullptr;
         a.max_price = max_price ? ln.p_max_price.p : nullptr; a.cloud = cloud ? ln.p_cloud.p : nullptr;
         a.P = nb;
-        fill_offer_args(ds, a);
+        fill_offer_args(ds.main, a);
         PersistPlan pl; bool persist = false;
-        const int R = prepare_select_scratch(ds, ln, nb, a, &pl, &persist);
+        const int R = prepare_select_scratch(ds, ds.main, ln, nb, a, &pl, &persist);
         for (int o = 0; o < n; ++o) a.best_out[o] = ctx->devs[(size_t)o].best_full.p;
         a.n_out = n; a.row0 = b0; a.top5 = top5 ? ln.top5.p : nullptr;
         a.self_out = s;  // own vector; finished push blocks / sub-batches are forwarded to the peers
@@ -442,8 +442,11 @@ void rpk_destroy(rpk_ctx* ctx) {
         if (ds.stream) cudaStreamSynchronize(ds.stream);
         ds.raw_mem.release(); ds.raw_vcpu.release(); ds.raw_ram.release(); ds.raw_sp.release(); ds.raw_cp.release(); ds.raw_flags.release();
         ds.sort_keys.release(); ds.sort_vals.release();
-        for (int c = 0; c < 2; ++c) { ds.v_bitmap[c].release(); ds.v_packed[c].release(); ds.v_wide[c].release(); ds.v_price[c].release(); ds.v_perm[c].release(); }
-        for (int d = 0; d < 3; ++d) ds.distinct[d].release();
+        ds.main.release();
+        for (auto& t : ds.sets) t.release();
+        ds.sets.clear();
+        ds.set_words.release(); ds.set_members.release(); ds.set_mem.release(); ds.set_vcpu.release(); ds.set_ram.release();
+        ds.set_sp.release(); ds.set_cp.release(); ds.set_flags.release(); ds.ss.release();
         ds.dcount.release();
         for (auto& ln : ds.lane) {
             if (ln.stream) cudaStreamSynchronize(ln.stream);
@@ -478,6 +481,7 @@ int rpk_offers_upload(rpk_ctx* ctx, uint32_t G, const int32_t* mem_gb, const int
         for (auto& ds : ctx->devs) {
             RPK_CUDA(cudaSetDevice(ds.dev));
             ds.offers_ready = false;
+            ++ds.table_version;  // offer sets built on the previous table are stale from here on
             ds.force_kind = 0;
             // test hook (exercise every kernel on any table): consulted once per table upload, never on the select path
             if (const char* fk = getenv("RPK_FORCE_KERNEL")) {
@@ -499,13 +503,14 @@ int rpk_offers_upload(rpk_ctx* ctx, uint32_t G, const int32_t* mem_gb, const int
                 RPK_CUDA(cudaMemcpyAsync(ds.raw_flags.p, flags, (size_t)G, cudaMemcpyHostToDevice, ds.stream));
             }
             OfferIngest in{G, ds.raw_mem.p, ds.raw_vcpu.p, ds.raw_ram.p, ds.raw_sp.p, ds.raw_cp.p, ds.raw_flags.p};
-            ctx->launches += (uint64_t)launch_offer_ingest(ds, in, ds.stream);
+            ctx->launches += (uint64_t)launch_offer_ingest(ds, ds.main, in, ds.stream);
             RPK_CUDA(cudaStreamSynchronize(ds.stream));
+            ds.offers_ready = true;
         }
         const DeviceState& d0 = ctx->devs[0];
-        ctx->stats.select_kernel_kind = d0.pk.bm_words ? 4u : d0.pk.bits ? (d0.pk.pos_bits ? 3u : 2u) : 1u;
-        ctx->stats.distinct_mem = d0.D[0]; ctx->stats.distinct_vcpu = d0.D[1]; ctx->stats.distinct_ram = d0.D[2];
-        ctx->stats.packed_bits = d0.pk.bits;
+        ctx->stats.select_kernel_kind = d0.main.pk.bm_words ? 4u : d0.main.pk.bits ? (d0.main.pk.pos_bits ? 3u : 2u) : 1u;
+        ctx->stats.distinct_mem = d0.main.D[0]; ctx->stats.distinct_vcpu = d0.main.D[1]; ctx->stats.distinct_ram = d0.main.D[2];
+        ctx->stats.packed_bits = d0.main.pk.bits;
         return RPK_OK;
     });
 }
@@ -525,9 +530,9 @@ int rpk_select_device_gather(rpk_ctx* ctx, int shard, uint32_t P, const int32_t*
         SelectArgs a{};
         a.req_mem = d_req_mem_gb; a.req_vcpu = d_req_vcpu; a.req_ram = d_req_ram_gb; a.max_price = d_max_price; a.cloud = d_cloud;
         a.P = P;
-        fill_offer_args(ds, a);
+        fill_offer_args(ds.main, a);
         PersistPlan pl; bool persist = false;
-        const int R = prepare_select_scratch(ds, ds.lane[0], P, a, &pl, &persist);
+        const int R = prepare_select_scratch(ds, ds.main, ds.lane[0], P, a, &pl, &persist);
         for (int o = 0; o < n_out; ++o) a.best_out[o] = d_best_full[o];
         a.n_out = n_out; a.row0 = row0; a.top5 = d_top5;
         a.self_out = find_local_vector(ctx, shard, ds.dev, n_out, d_best_full);
@@ -537,7 +542,7 @@ int rpk_select_device_gather(rpk_ctx* ctx, int shard, uint32_t P, const int32_t*
         ctx->launches += (uint64_t)run_select(ds.lane[0], a, R, persist ? &pl : nullptr, st);
         guard.done();
         ctx->stats.select_calls += 1;
-        ctx->stats.offer_scores += (uint64_t)P * ds.G;
+        ctx->stats.offer_scores += (uint64_t)P * ds.main.G;
         return RPK_OK;
     });
 }
@@ -561,7 +566,7 @@ int rpk_select(rpk_ctx* ctx, uint32_t P, const int32_t* req_mem_gb, const int32_
             int rc = select_small(ctx, ctx->devs[0], P, req_mem_gb, req_vcpu, req_ram_gb, max_price, cloud, best, top5, &ctx->launches);
             ctx->stats.last_select_kernel_ms = 0.f; ctx->stats.last_select_total_ms = 0.f;
             ctx->stats.select_calls += 1;
-            ctx->stats.offer_scores += (uint64_t)P * ctx->devs[0].G;
+            ctx->stats.offer_scores += (uint64_t)P * ctx->devs[0].main.G;
             return rc;
         }
         std::vector<uint64_t> launches((size_t)n, 0);
@@ -578,7 +583,189 @@ int rpk_select(rpk_ctx* ctx, uint32_t P, const int32_t* req_mem_gb, const int32_
         ctx->stats.last_select_kernel_ms = 0.f;  // copies and kernels overlap in the pipelined host path: only the total is meaningful
         ctx->stats.last_select_total_ms = tmax;
         ctx->stats.select_calls += 1;
-        ctx->stats.offer_scores += (uint64_t)P * ctx->devs[0].G;
+        ctx->stats.offer_scores += (uint64_t)P * ctx->devs[0].main.G;
+        return RPK_OK;
+    });
+}
+
+// ---- offer sets --------------------------------------------------------------------------------------------
+
+int rpk_offer_sets_upload(rpk_ctx* ctx, uint32_t n_sets, uint32_t G, const uint32_t* members) {
+    if (!ctx) return RPK_EINVAL;
+    if (n_sets > RPK_MAX_OFFER_SETS) return fail(ctx, RPK_EINVAL, "rpk_offer_sets_upload: at most RPK_MAX_OFFER_SETS (256) sets");
+    for (auto& ds : ctx->devs) if (!ds.offers_ready) return fail(ctx, RPK_ESTATE, "rpk_offer_sets_upload: no offer table uploaded (call rpk_offers_upload first)");
+    if (G != ctx->devs[0].main.G) return fail(ctx, RPK_EINVAL, "rpk_offer_sets_upload: G differs from the resident offer table's");
+    const uint32_t W = (G + 31) / 32;
+    if (n_sets > 0 && W > 0 && !members) return fail(ctx, RPK_EINVAL, "rpk_offer_sets_upload: members is NULL");
+    // member counts from the words themselves (bits >= G ignored): the host sizes every sub-table without a readback
+    std::vector<uint32_t> counts(n_sets, 0);
+    for (uint32_t s = 0; s < n_sets; ++s) {
+        uint32_t c = 0;
+        for (uint32_t w = 0; w < W; ++w) {
+            uint32_t m = members[(size_t)s * W + w];
+            if ((w + 1) * 32 > G) m &= (1u << (G - w * 32)) - 1u;
+            c += (uint32_t)__builtin_popcount(m);
+        }
+        counts[s] = c;
+    }
+    return guarded(ctx, [&]() -> int {
+        for (auto& ds : ctx->devs) {
+            RPK_CUDA(cudaSetDevice(ds.dev));
+            ds.sets_ready = false;
+            for (size_t s = n_sets; s < ds.sets.size(); ++s) ds.sets[s].release();
+            ds.sets.resize(n_sets);
+            if (n_sets && W) {
+                ds.set_words.reserve((size_t)n_sets * W);
+                RPK_CUDA(cudaMemcpyAsync(ds.set_words.p, members, (size_t)n_sets * W * 4, cudaMemcpyHostToDevice, ds.stream));
+            }
+            ctx->launches += (uint64_t)launch_offer_sets_build(ds, n_sets, ds.set_words.p, counts.data(), ds.stream);
+            RPK_CUDA(cudaStreamSynchronize(ds.stream));
+            ds.sets_ready = true;
+            ds.sets_version = ds.table_version;
+        }
+        return RPK_OK;
+    });
+}
+
+namespace {
+
+struct SetCols {  // one shard's pod columns on its device (nullable ones as in rpk_select)
+    const int32_t* mem; const int32_t* vcpu; const int32_t* ram; const double* price; const uint8_t* cloud; const uint16_t* set_id;
+};
+
+int check_sets_state(rpk_ctx* ctx, const DeviceState& ds) {
+    if (!ds.offers_ready) return fail(ctx, RPK_ESTATE, "rpk_select_sets: no offer table uploaded (call rpk_offers_upload first)");
+    if (!ds.sets_ready || ds.sets_version != ds.table_version)
+        return fail(ctx, RPK_ESTATE, "rpk_select_sets: no offer sets for the current offer table (call rpk_offer_sets_upload after rpk_offers_upload)");
+    return RPK_OK;
+}
+
+// One shard's restricted select on stream st: partition the rows by set id, one select per non-empty bin against its
+// set's sub-table (lane 0's scratch, one bin after the other), write-back in row order.  Synchronises st once (the bin
+// counts); with no set column it is one plain select against the resident table.  *scores += sum of P_s * G_s.
+void select_sets_shard(DeviceState& ds, uint32_t P, const SetCols& c, int32_t* d_best, int32_t* d_top5, cudaStream_t st,
+                       uint64_t* launches, uint64_t* scores) {
+    DeviceState::Lane& ln = ds.lane[0];
+    auto select_on = [&](const OfferTable& t, uint32_t n, const int32_t* m, const int32_t* v, const int32_t* r, const double* pr,
+                         const uint8_t* cl, int32_t* best_vec, uint32_t row0, int32_t* top5) {
+        SelectArgs a{};
+        a.req_mem = m; a.req_vcpu = v; a.req_ram = r; a.max_price = pr; a.cloud = cl;
+        a.P = n;
+        fill_offer_args(t, a);
+        PersistPlan pl; bool persist = false;
+        const int R = prepare_select_scratch(ds, t, ln, n, a, &pl, &persist);
+        a.best_out[0] = best_vec; a.n_out = 1; a.self_out = 0; a.row0 = row0; a.top5 = top5;
+        *launches += (uint64_t)run_select(ln, a, R, persist ? &pl : nullptr, st);
+        *scores += (uint64_t)n * t.G;
+    };
+    if (!c.set_id) { select_on(ds.main, P, c.mem, c.vcpu, c.ram, c.price, c.cloud, d_best, 0, d_top5); return; }
+    const uint32_t n_sets = (uint32_t)ds.sets.size(), nb = n_sets + 2;
+    DeviceState::SetSelect& ss = ds.ss;
+    ss.p_mem.reserve(P); ss.rows.reserve(P); ss.tmp_best.reserve(P); ss.hist.reserve(2 * (RPK_MAX_OFFER_SETS + 2));
+    if (c.vcpu) ss.p_vcpu.reserve(P);
+    if (c.ram) ss.p_ram.reserve(P);
+    if (c.price) ss.p_price.reserve(P);
+    if (c.cloud) ss.p_cloud.reserve(P);
+    if (d_top5) ss.tmp_top5.reserve((size_t)P * RPK_TOPK);
+    if (!ss.h_counts) RPK_CUDA(cudaHostAlloc((void**)&ss.h_counts, (RPK_MAX_OFFER_SETS + 2) * sizeof(uint32_t), cudaHostAllocPortable));
+    RPK_CUDA(cudaMemsetAsync(ss.hist.p, 0, (size_t)2 * nb * sizeof(uint32_t), st));
+    SetPartitionArgs pa{};
+    pa.P = P; pa.n_sets = n_sets; pa.set_id = c.set_id;
+    pa.req_mem = c.mem; pa.req_vcpu = c.vcpu; pa.req_ram = c.ram; pa.max_price = c.price; pa.cloud = c.cloud;
+    pa.o_mem = ss.p_mem.p; pa.o_vcpu = ss.p_vcpu.p; pa.o_ram = ss.p_ram.p; pa.o_price = ss.p_price.p; pa.o_cloud = ss.p_cloud.p;
+    pa.rows = ss.rows.p; pa.hist = ss.hist.p;
+    *launches += (uint64_t)launch_set_partition(pa, st);
+    RPK_CUDA(cudaMemcpyAsync(ss.h_counts, ss.hist.p, (size_t)nb * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    RPK_CUDA(cudaStreamSynchronize(st));  // the one synchronisation: bin sizes decide the launches below
+    uint32_t start = 0;
+    for (uint32_t b = 0; b < nb; ++b) {
+        const uint32_t cnt = ss.h_counts[b];
+        if (cnt == 0) continue;
+        const OfferTable* t = b < n_sets ? &ds.sets[b] : b == n_sets ? &ds.main : nullptr;
+        int32_t* t5 = d_top5 ? ss.tmp_top5.p + (size_t)start * RPK_TOPK : nullptr;
+        if (t && t->G) {
+            select_on(*t, cnt, ss.p_mem.p + start, c.vcpu ? ss.p_vcpu.p + start : nullptr, c.ram ? ss.p_ram.p + start : nullptr,
+                      c.price ? ss.p_price.p + start : nullptr, c.cloud ? ss.p_cloud.p + start : nullptr, ss.tmp_best.p, start, t5);
+        } else {  // empty set or unknown id: nothing is feasible
+            RPK_CUDA(cudaMemsetAsync(ss.tmp_best.p + start, 0xFF, (size_t)cnt * 4, st));
+            if (t5) RPK_CUDA(cudaMemsetAsync(t5, 0xFF, (size_t)cnt * RPK_TOPK * 4, st));
+        }
+        start += cnt;
+    }
+    *launches += (uint64_t)launch_set_unpermute(P, ss.rows.p, ss.tmp_best.p, d_top5 ? ss.tmp_top5.p : nullptr, d_best, d_top5, st);
+}
+
+}  // namespace
+
+int rpk_select_sets_device(rpk_ctx* ctx, int shard, uint32_t P, const int32_t* d_req_mem_gb, const int32_t* d_req_vcpu,
+                           const int32_t* d_req_ram_gb, const double* d_max_price, const uint8_t* d_cloud,
+                           const uint16_t* d_set_id, int32_t* d_best, int32_t* d_top5, void* stream) {
+    if (!ctx) return RPK_EINVAL;
+    if (shard < 0 || (size_t)shard >= ctx->devs.size()) return fail(ctx, RPK_EINVAL, "rpk_select_sets_device: shard out of range");
+    if (P == 0) return RPK_OK;
+    if (!d_req_mem_gb || !d_best) return fail(ctx, RPK_EINVAL, "rpk_select_sets_device: req_mem_gb and best are required");
+    DeviceState& ds = ctx->devs[(size_t)shard];
+    if (!ds.offers_ready) return fail(ctx, RPK_ESTATE, "rpk_select_sets: no offer table uploaded (call rpk_offers_upload first)");
+    if (d_set_id) { if (int rc = check_sets_state(ctx, ds)) return rc; }
+    return guarded(ctx, [&]() -> int {
+        RPK_CUDA(cudaSetDevice(ds.dev));
+        cudaStream_t st = stream ? (cudaStream_t)stream : ds.stream;
+        if (d_set_id) {  // the bin counts are read back mid-call: refuse a capturing stream before enqueuing anything
+            cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+            RPK_CUDA(cudaStreamIsCapturing(st, &cs));
+            if (cs != cudaStreamCaptureStatusNone)
+                return fail(ctx, RPK_ESTATE, "rpk_select_sets_device: the stream is being captured; with set ids the call synchronises it once and cannot be captured");
+        }
+        ScratchGuard guard(&ds.sel_last_stream, ds.ev_sel, st);
+        uint64_t scores = 0;
+        const SetCols c{d_req_mem_gb, d_req_vcpu, d_req_ram_gb, d_max_price, d_cloud, d_set_id};
+        select_sets_shard(ds, P, c, d_best, d_top5, st, &ctx->launches, &scores);
+        guard.done();
+        ctx->stats.select_calls += 1;
+        ctx->stats.offer_scores += scores;
+        return RPK_OK;
+    });
+}
+
+int rpk_select_sets(rpk_ctx* ctx, uint32_t P, const int32_t* req_mem_gb, const int32_t* req_vcpu, const int32_t* req_ram_gb,
+                    const double* max_price, const uint8_t* cloud, const uint16_t* set_id, int32_t* best, int32_t* top5) {
+    if (!ctx) return RPK_EINVAL;
+    if (P == 0) return RPK_OK;
+    if (!req_mem_gb || !best) return fail(ctx, RPK_EINVAL, "rpk_select_sets: req_mem_gb and best are required");
+    for (auto& ds : ctx->devs) {
+        if (!ds.offers_ready) return fail(ctx, RPK_ESTATE, "rpk_select_sets: no offer table uploaded (call rpk_offers_upload first)");
+        if (set_id) { if (int rc = check_sets_state(ctx, ds)) return rc; }
+    }
+    return guarded(ctx, [&]() -> int {
+        const int n = (int)ctx->devs.size();
+        std::vector<uint64_t> launches((size_t)n, 0), scores((size_t)n, 0);
+        // rows are sharded like rpk_select's; each shard is one sub-batch: H2D, partition + selects, D2H
+        ctx->workers.run(n, [&](int s) {
+            DeviceState& ds = ctx->devs[(size_t)s];
+            uint32_t lo, hi; shard_range(P, n, s, &lo, &hi);
+            const uint32_t Ps = hi - lo;
+            if (Ps == 0) return;
+            RPK_CUDA(cudaSetDevice(ds.dev));
+            DeviceState::SetSelect& ss = ds.ss;
+            cudaStream_t st = ds.stream;
+            ScratchGuard guard(&ds.sel_last_stream, ds.ev_sel, st);
+            ss.in_mem.reserve(Ps); ss.out_best.reserve(Ps);
+            RPK_CUDA(cudaMemcpyAsync(ss.in_mem.p, req_mem_gb + lo, (size_t)Ps * 4, cudaMemcpyHostToDevice, st));
+            SetCols c{ss.in_mem.p, nullptr, nullptr, nullptr, nullptr, nullptr};
+            if (req_vcpu) { ss.in_vcpu.reserve(Ps); RPK_CUDA(cudaMemcpyAsync(ss.in_vcpu.p, req_vcpu + lo, (size_t)Ps * 4, cudaMemcpyHostToDevice, st)); c.vcpu = ss.in_vcpu.p; }
+            if (req_ram_gb) { ss.in_ram.reserve(Ps); RPK_CUDA(cudaMemcpyAsync(ss.in_ram.p, req_ram_gb + lo, (size_t)Ps * 4, cudaMemcpyHostToDevice, st)); c.ram = ss.in_ram.p; }
+            if (max_price) { ss.in_price.reserve(Ps); RPK_CUDA(cudaMemcpyAsync(ss.in_price.p, max_price + lo, (size_t)Ps * 8, cudaMemcpyHostToDevice, st)); c.price = ss.in_price.p; }
+            if (cloud) { ss.in_cloud.reserve(Ps); RPK_CUDA(cudaMemcpyAsync(ss.in_cloud.p, cloud + lo, (size_t)Ps, cudaMemcpyHostToDevice, st)); c.cloud = ss.in_cloud.p; }
+            if (set_id) { ss.in_set.reserve(Ps); RPK_CUDA(cudaMemcpyAsync(ss.in_set.p, set_id + lo, (size_t)Ps * 2, cudaMemcpyHostToDevice, st)); c.set_id = ss.in_set.p; }
+            if (top5) ss.out_top5.reserve((size_t)Ps * RPK_TOPK);
+            select_sets_shard(ds, Ps, c, ss.out_best.p, top5 ? ss.out_top5.p : nullptr, st, &launches[(size_t)s], &scores[(size_t)s]);
+            RPK_CUDA(cudaMemcpyAsync(best + lo, ss.out_best.p, (size_t)Ps * 4, cudaMemcpyDeviceToHost, st));
+            if (top5) RPK_CUDA(cudaMemcpyAsync(top5 + (size_t)lo * RPK_TOPK, ss.out_top5.p, (size_t)Ps * RPK_TOPK * 4, cudaMemcpyDeviceToHost, st));
+            guard.done();
+            RPK_CUDA(cudaStreamSynchronize(st));
+        });
+        for (int s = 0; s < n; ++s) { ctx->launches += launches[(size_t)s]; ctx->stats.offer_scores += scores[(size_t)s]; }
+        ctx->stats.select_calls += 1;
         return RPK_OK;
     });
 }
@@ -931,7 +1118,7 @@ int rpk_tick(rpk_ctx* ctx, uint32_t P, const int32_t* req_mem_gb, const int32_t*
         for (int s = 0; s < n; ++s) { total += collect_status_shard(ctx, s, h, total); ctx->launches += launches[(size_t)s]; }
         *n_changed = total;
         ctx->stats.status_calls += 1; ctx->stats.status_records += N;
-        if (P > 0) { ctx->stats.select_calls += 1; ctx->stats.offer_scores += (uint64_t)P * ctx->devs[0].G; }
+        if (P > 0) { ctx->stats.select_calls += 1; ctx->stats.offer_scores += (uint64_t)P * ctx->devs[0].main.G; }
         return RPK_OK;
     });
 }

@@ -146,7 +146,23 @@ struct OfferIngest {   // raw device columns in, views out
 };
 
 struct DeviceState;
-int launch_offer_ingest(DeviceState& ds, const OfferIngest& in, cudaStream_t st);
+struct OfferTable;
+int launch_offer_ingest(DeviceState& ds, OfferTable& t, const OfferIngest& in, cudaStream_t st);
+// offer sets (offers.cu): member lists of n_sets sets from their membership words (W = ceil(G/32) per set) and one
+// sub-table per non-empty set; counts[s] = members of set s (computed by the caller from the same words)
+int launch_offer_sets_build(DeviceState& ds, uint32_t n_sets, const uint32_t* d_words, const uint32_t* counts, cudaStream_t st);
+// offer sets (sets.cu): partition of pod rows by set id and the write-back in row order
+struct SetPartitionArgs {
+    uint32_t P, n_sets;             // bins: 0..n_sets-1 the sets, n_sets = RPK_SET_ALL, n_sets+1 = out of range
+    const uint16_t* set_id;
+    const int32_t* req_mem; const int32_t* req_vcpu; const int32_t* req_ram; const double* max_price; const uint8_t* cloud;
+    int32_t* o_mem; int32_t* o_vcpu; int32_t* o_ram; double* o_price; uint8_t* o_cloud;  // partitioned copies (present columns)
+    uint32_t* rows;                 // [P] row id of partitioned position i
+    uint32_t* hist;                 // [n_sets + 2] rows per bin, then [n_sets + 2] write cursors (zeroed by the caller)
+};
+int launch_set_partition(const SetPartitionArgs& a, cudaStream_t st);
+int launch_set_unpermute(uint32_t P, const uint32_t* rows, const int32_t* tmp_best, const int32_t* tmp_top5, int32_t* best,
+                         int32_t* top5, cudaStream_t st);
 struct PersistPlan;
 int launch_select(const SelectArgs& a, int rows_per_warp, const PersistPlan* pl, cudaStream_t st);
 uint32_t select_tiles_max(uint32_t P, int rows_per_warp);
@@ -182,21 +198,56 @@ struct DevBuf {  // grow-only device buffer
     void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
 };
 
+// The views of one offer table as the select kernels consume them: the resident table, or the sub-table of an offer
+// set (whose perm / wide.w hold global offer ids, so the kernels emit global indices directly).
+struct OfferTable {
+    uint32_t G = 0, Gpad = 0;
+    DevBuf<uint32_t> v_packed[2]; DevBuf<uint32_t> v_bitmap[2]; DevBuf<uint32_t> v_bitmapT[2]; uint32_t nsub = 0; DevBuf<int4> v_wide[2]; DevBuf<double> v_price[2]; DevBuf<int32_t> v_perm[2];
+    DevBuf<int32_t> distinct[3];
+    uint32_t D[3] = {0, 0, 0};
+    PackLayout pk = {};
+    void release() {
+        for (int c = 0; c < 2; ++c) { v_packed[c].release(); v_bitmap[c].release(); v_bitmapT[c].release(); v_wide[c].release(); v_price[c].release(); v_perm[c].release(); }
+        for (int d = 0; d < 3; ++d) distinct[d].release();
+        G = Gpad = nsub = 0;
+    }
+};
+
 struct DeviceState {
     int dev = -1;
     int sm_count = 148;
     cudaStream_t stream = nullptr;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
     // offer table
-    uint32_t G = 0, Gpad = 0;
+    OfferTable main;
     bool offers_ready = false;
+    uint64_t table_version = 0;  // bumped by every rpk_offers_upload
     DevBuf<int32_t> raw_mem, raw_vcpu, raw_ram; DevBuf<double> raw_sp, raw_cp; DevBuf<uint8_t> raw_flags;
-    DevBuf<unsigned long long> sort_keys; DevBuf<uint32_t> sort_vals;
-    DevBuf<uint32_t> v_packed[2]; DevBuf<uint32_t> v_bitmap[2]; DevBuf<uint32_t> v_bitmapT[2]; uint32_t nsub = 0; DevBuf<int4> v_wide[2]; DevBuf<double> v_price[2]; DevBuf<int32_t> v_perm[2];
-    DevBuf<int32_t> distinct[3]; DevBuf<uint32_t> dcount;
-    uint32_t D[3] = {0, 0, 0};
-    PackLayout pk = {};
+    DevBuf<unsigned long long> sort_keys; DevBuf<uint32_t> sort_vals;  // shared by every ingest (resident table and sets)
+    DevBuf<uint32_t> dcount;
     int force_kind = 0;  // RPK_FORCE_KERNEL (tests): 0 auto, 1 generic, 2 packed+select, 3 packed+pos, 4 bit-sliced
+    // offer sets: one sub-table per set (G = 0 for an empty set: never selected against), valid while
+    // sets_version == table_version
+    std::vector<OfferTable> sets;
+    bool sets_ready = false;
+    uint64_t sets_version = 0;
+    DevBuf<uint32_t> set_words, set_members;  // membership words as uploaded; ascending member lists, set after set
+    DevBuf<int32_t> set_mem, set_vcpu, set_ram; DevBuf<double> set_sp, set_cp; DevBuf<uint8_t> set_flags;  // gathered raw columns
+    // rpk_select_sets scratch: partitioned pod columns, row ids, bin counts, results in partitioned order; host path staging
+    struct SetSelect {
+        DevBuf<int32_t> p_mem, p_vcpu, p_ram; DevBuf<double> p_price; DevBuf<uint8_t> p_cloud;
+        DevBuf<uint32_t> rows, hist; DevBuf<int32_t> tmp_best, tmp_top5;
+        DevBuf<int32_t> in_mem, in_vcpu, in_ram; DevBuf<double> in_price; DevBuf<uint8_t> in_cloud; DevBuf<uint16_t> in_set;
+        DevBuf<int32_t> out_best, out_top5;
+        uint32_t* h_counts = nullptr;  // pinned: bin counts read back once per call
+        void release() {
+            p_mem.release(); p_vcpu.release(); p_ram.release(); p_price.release(); p_cloud.release(); rows.release(); hist.release();
+            tmp_best.release(); tmp_top5.release(); in_mem.release(); in_vcpu.release(); in_ram.release(); in_price.release();
+            in_cloud.release(); in_set.release(); out_best.release(); out_top5.release();
+            if (h_counts) cudaFreeHost(h_counts);
+            h_counts = nullptr;
+        }
+    } ss;
     // select scratch.  The host entry point pipelines row sub-batches over four lanes (stream + staging +
     // scratch each) so that the H2D of one sub-batch, the kernels of another and the D2H of a third overlap;
     // the device entry points use lane 0's scratch on the caller's stream.

@@ -39,6 +39,20 @@ def _dev_ptr(t, dtype_name, n=None, name="tensor"):
     return C.c_void_p(t.data_ptr())
 
 
+def pack_offer_sets(members) -> np.ndarray:
+    """bool ``(n_sets, G)`` -> uint32 ``(n_sets, ceil(G/32))`` membership words of rpk_offer_sets_upload: offer g of set
+    s is bit ``g & 31`` of word ``g // 32`` (little-endian bit and byte order)."""
+    m = np.asarray(members, dtype=bool)
+    if m.ndim != 2:
+        raise ValueError("members: expected a (n_sets, G) bool array")
+    n_sets, G = m.shape
+    W = (G + 31) // 32
+    b = np.packbits(m, axis=1, bitorder="little")
+    out = np.zeros((n_sets, W * 4), np.uint8)
+    out[:, : b.shape[1]] = b
+    return np.ascontiguousarray(out.view("<u4").astype(np.uint32, copy=False))
+
+
 class Engine:
     """One ``rpk_ctx``.  ``n_gpus > 1`` = one process driving several GPUs (the Go kubelet's shape)."""
 
@@ -134,6 +148,43 @@ class Engine:
             _dev_ptr(pods.get("req_ram_gb"), "int32", P), _dev_ptr(pods.get("max_price"), "float64", P),
             _dev_ptr(pods.get("cloud"), "uint8", P), len(full_ptrs), arr, row0, _dev_ptr(d_top5, "int32", P * 5),
             C.c_void_p(st)))
+
+    # -- offer sets ----------------------------------------------------------------------------------------
+    def upload_offer_sets(self, members):
+        """``members``: bool ``(n_sets, G)`` -- row s marks the offers of set s (``G`` = the resident table's).
+        Replaces every previous set; ``n_sets = 0`` clears them (rpk_offer_sets_upload)."""
+        words = pack_offer_sets(members)
+        n_sets, G = np.asarray(members).shape
+        self._check(self._lib.rpk_offer_sets_upload(self._ctx, n_sets, G, C.c_void_p(words.ctypes.data) if words.size else None))
+
+    def select_sets(self, pods: dict, set_id, want_top5: bool = False):
+        """``select`` with every row restricted to offer set ``set_id[p]`` (uint16; ``RPK_SET_ALL`` = the whole table,
+        ``None`` = every row unrestricted).  -> ``(best[P], top5[P,5] | None)``"""
+        P = int(pods["req_mem_gb"].shape[0])
+        best = np.empty(P, np.int32)
+        top5 = np.empty((P, 5), np.int32) if want_top5 else None
+        self._check(self._lib.rpk_select_sets(
+            self._ctx, P, _np_ptr(pods["req_mem_gb"], np.int32, P, "req_mem_gb"), _np_ptr(pods.get("req_vcpu"), np.int32, P, "req_vcpu"),
+            _np_ptr(pods.get("req_ram_gb"), np.int32, P, "req_ram_gb"), _np_ptr(pods.get("max_price"), np.float64, P, "max_price"),
+            _np_ptr(pods.get("cloud"), np.uint8, P, "cloud"), _np_ptr(set_id, np.uint16, P, "set_id"), _np_ptr(best, np.int32, P, "best"),
+            _np_ptr(top5, np.int32, P * 5, "top5") if top5 is not None else None))
+        return best, top5
+
+    def select_sets_device(self, pods: dict, d_set_id, d_best, d_top5=None, shard: int = 0, stream=None):
+        """torch CUDA columns in (``d_set_id`` int16 holding the uint16 ids, or None), results enqueued on ``stream``;
+        the call synchronises the stream once to read the per-set row counts."""
+        import torch
+
+        P = int(pods["req_mem_gb"].numel())
+        st = stream if stream is not None else (torch.cuda.current_stream().cuda_stream or 1)  # 0 -> cudaStreamLegacy
+        if d_set_id is not None and (not d_set_id.is_cuda or d_set_id.element_size() != 2 or not d_set_id.is_contiguous()
+                                     or d_set_id.numel() != P):
+            raise TypeError("d_set_id: expected a contiguous CUDA tensor of P 16-bit ids (torch.int16 / torch.uint16)")
+        self._check(self._lib.rpk_select_sets_device(
+            self._ctx, shard, P, _dev_ptr(pods["req_mem_gb"], "int32", P), _dev_ptr(pods.get("req_vcpu"), "int32", P),
+            _dev_ptr(pods.get("req_ram_gb"), "int32", P), _dev_ptr(pods.get("max_price"), "float64", P),
+            _dev_ptr(pods.get("cloud"), "uint8", P), C.c_void_p(d_set_id.data_ptr()) if d_set_id is not None else None,
+            _dev_ptr(d_best, "int32", P), _dev_ptr(d_top5, "int32", P * 5), C.c_void_p(st)))
 
     # -- cross-process peer vectors (CUDA IPC) ------------------------------------------------------------
     def ipc_alloc(self, nbytes: int, shard: int = 0):

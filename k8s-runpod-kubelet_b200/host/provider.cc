@@ -85,6 +85,19 @@ static std::string TrimSpace(const std::string& s) {
     return s.substr(a, b - a);
 }
 
+std::vector<std::string> ParseGpuTypeIds(const std::string& v) {
+    std::vector<std::string> out;
+    if (v.empty()) return out;
+    size_t start = 0;
+    while (true) {  // strings.Split(v, ","): empty elements are kept ("a,,b" -> "a", "", "b"); they match no GPU type
+        const size_t comma = v.find(',', start);
+        out.push_back(TrimSpace(v.substr(start, comma == std::string::npos ? std::string::npos : comma - start)));
+        if (comma == std::string::npos) break;
+        start = comma + 1;
+    }
+    return out;
+}
+
 // GetRequestedPorts -- runpod_client.go:1381-1393 (the pod-spec half, extractPortsFromPod :1195-1246, is the
 // caller's: Pod::container_ports already holds "port/protocol" strings)
 std::vector<std::string> GetRequestedPorts(const Pod& pod) {
@@ -212,26 +225,28 @@ static int32_t ClampI32(long long v) { return v > INT32_MAX ? INT32_MAX : v < IN
 // reference-shaped functions (GetAnnotationWithFallback / ValidateCloudType / ExtractGPUMemory).
 namespace {
 const std::string kKeyCloud = CloudTypeAnnotation, kKeyMem = GpuMemoryAnnotation, kKeyVcpu = VcpuAnnotation,
-                  kKeyRam = RamAnnotation, kKeyMaxPrice = MaxPriceAnnotation;
+                  kKeyRam = RamAnnotation, kKeyMaxPrice = MaxPriceAnnotation, kKeyGpuTypes = GpuTypeIdsAnnotation;
 
-// The five annotations the row reads.  One pass over the pod's annotation map (and one over the owner Job's, if a
+// The six annotations the row reads.  One pass over the pod's annotation map (and one over the owner Job's, if a
 // slot is still open) classifies each key by length + full compare, instead of five string-keyed tree searches
 // per map: per key the result is getAnnotationWithFallback's (:1102-1112) -- the pod's non-empty value, else the
 // Job's non-empty value, else nullptr (= the default).
-enum Slot { kSlotCloud, kSlotMem, kSlotVcpu, kSlotRam, kSlotMaxPrice, kSlots };
+enum Slot { kSlotCloud, kSlotMem, kSlotVcpu, kSlotRam, kSlotMaxPrice, kSlotGpuTypes, kSlots };
 constexpr size_t CLen(const char* s) { size_t n = 0; while (s[n]) ++n; return n; }
 static_assert(CLen(CloudTypeAnnotation) == 20 && CLen(GpuMemoryAnnotation) == 29 && CLen(VcpuAnnotation) == 23 &&
-              CLen(RamAnnotation) == 25 && CLen(MaxPriceAnnotation) == 26, "ClassifyKey switches on these lengths");
+              CLen(RamAnnotation) == 25 && CLen(MaxPriceAnnotation) == 26 && CLen(GpuTypeIdsAnnotation) == 22,
+              "ClassifyKey switches on these lengths");
 
 inline int ClassifyKey(const std::string& k) {
     const std::string* want = nullptr;
     int slot = kSlots;
-    switch (k.size()) {  // the five keys have five different lengths
+    switch (k.size()) {  // the six keys have six different lengths
         case 20: want = &kKeyCloud; slot = kSlotCloud; break;      // runpod.io/cloud-type  (runpod.io/templateId is 20 too)
         case 29: want = &kKeyMem; slot = kSlotMem; break;          // runpod.io/required-gpu-memory
         case 23: want = &kKeyVcpu; slot = kSlotVcpu; break;        // runpod.io/required-vcpu
         case 25: want = &kKeyRam; slot = kSlotRam; break;          // runpod.io/required-ram-gb
         case 26: want = &kKeyMaxPrice; slot = kSlotMaxPrice; break;  // runpod.io/max-price-per-hr
+        case 22: want = &kKeyGpuTypes; slot = kSlotGpuTypes; break;  // runpod.io/gpu-type-ids
         default: return kSlots;
     }
     return k == *want ? slot : (int)kSlots;
@@ -250,7 +265,7 @@ inline void CollectAnnotations(const Pod& pod, const std::string* (&v)[kSlots]) 
     }
 }
 
-struct Row { int32_t mem, vcpu, ram; double max_price; uint8_t cloud; };
+struct Row { int32_t mem, vcpu, ram; double max_price; uint8_t cloud; const std::string* gpu_types; };
 
 Row PrepareRow(const Pod& pod) {
     const std::string* a[kSlots];
@@ -275,6 +290,7 @@ Row PrepareRow(const Pod& pod) {
         const double d = std::strtod(v->c_str(), &end);
         if (errno == 0 && end && *end == '\0' && end != v->c_str()) r.max_price = d;
     }
+    r.gpu_types = a[kSlotGpuTypes];  // nullptr: unrestricted
     return r;
 }
 }  // namespace
@@ -284,6 +300,8 @@ PodColumns PrepareColumns(const Pod& pod) {
     PodColumns c;
     c.req_mem_gb = r.mem; c.req_vcpu = r.vcpu; c.req_ram_gb = r.ram; c.max_price = r.max_price; c.cloud = r.cloud;
     c.cloud_type = r.cloud == RPK_CLOUD_COMMUNITY ? "COMMUNITY" : "SECURE";
+    c.restricted = r.gpu_types != nullptr;
+    if (r.gpu_types) c.gpu_type_ids = ParseGpuTypeIds(*r.gpu_types);
     return c;
 }
 
@@ -295,6 +313,7 @@ void PrepareColumnsBatch(const std::vector<PodPtr>& pods, PodColumnsSoA* out, in
             const Row r = PrepareRow(*pods[i]);
             out->req_mem_gb[i] = r.mem; out->req_vcpu[i] = r.vcpu; out->req_ram_gb[i] = r.ram;
             out->max_price[i] = r.max_price; out->cloud[i] = r.cloud;
+            if (r.gpu_types) out->gpu_type_ids[i] = *r.gpu_types;
         }
     };
     constexpr size_t kMinRowsPerThread = 4096;  // below this a thread costs more to start than it saves
@@ -549,9 +568,15 @@ bool Provider::DeployBatch(const std::vector<std::string>& keys) {
         // between the select and the lookup (indices would resolve against a different, possibly shorter, table)
         std::lock_guard<std::mutex> g(engine_mutex_);
         if (!RefreshOffersLocked(&err)) return false;  // "failed to get GPU types": every pod of the batch retries later
-        if (rpk_select(ctx_, P, cols.req_mem_gb.data(), cols.req_vcpu.data(), cols.req_ram_gb.data(), cols.max_price.data(),
-                       cols.cloud.data(), best.data(), top5.data()) != RPK_OK) return false;
-        ++select_calls_;
+        bool restricted = false;
+        for (uint32_t i = 0; i < P && !restricted; ++i) restricted = !cols.gpu_type_ids[i].empty();
+        if (!restricted) {  // no pod carries runpod.io/gpu-type-ids: the plain selection, exactly as without the annotation
+            if (rpk_select(ctx_, P, cols.req_mem_gb.data(), cols.req_vcpu.data(), cols.req_ram_gb.data(), cols.max_price.data(),
+                           cols.cloud.data(), best.data(), top5.data()) != RPK_OK) return false;
+            ++select_calls_;
+        } else if (!SelectWithSetsLocked(cols, top5.data()) && !(set_lists_.empty() && SelectWithSetsLocked(cols, top5.data(), false))) {
+            return false;  // a failed reuse forgets the resident sets and uploads once more; a second failure retries next tick
+        }
         for (uint32_t i = 0; i < P; ++i)
             for (int k = 0; k < RPK_TOPK; ++k) {
                 const int32_t g = top5[(size_t)i * RPK_TOPK + k];
@@ -575,6 +600,82 @@ bool Provider::DeployBatch(const std::vector<std::string>& keys) {
         it->second.info.ID = id; it->second.info.CostPerHr = cost;
     }
     return all_ok;
+}
+
+// A batch with runpod.io/gpu-type-ids: every distinct list, taken as a set of ids, becomes an offer set (ids absent from
+// the table are ignored, so a list that matches nothing is an empty set and its pods get an empty gpuTypeIds -- "no
+// eligible GPU types", retried like any other).  The resident sets are reused while the table is unchanged and hold
+// every list of the batch; otherwise the batch's lists are uploaded, RPK_MAX_OFFER_SETS at a time, each group with one
+// rpk_select_sets over its rows (the unrestricted rows go with the first group).  set_lists_ only names sets the engine
+// holds: it is cleared before an upload (a failed upload leaves none behind) and after a failed select on reused sets.
+bool Provider::SelectWithSetsLocked(const PodColumnsSoA& cols, int32_t* top5, bool may_reuse) {
+    const uint32_t P = (uint32_t)cols.size();
+    std::map<std::vector<std::string>, uint32_t> list_of;  // canonical list (sorted, unique ids) -> index in `lists`
+    std::vector<std::vector<std::string>> lists;
+    std::vector<uint32_t> row_list(P, UINT32_MAX);          // UINT32_MAX = unrestricted
+    for (uint32_t i = 0; i < P; ++i) {
+        if (cols.gpu_type_ids[i].empty()) continue;
+        std::vector<std::string> ids = ParseGpuTypeIds(cols.gpu_type_ids[i]);
+        std::sort(ids.begin(), ids.end());
+        ids.erase(std::unique(ids.begin(), ids.end()), ids.end());
+        auto it = list_of.emplace(std::move(ids), (uint32_t)lists.size());
+        if (it.second) lists.push_back(it.first->first);
+        row_list[i] = it.first->second;
+    }
+    std::map<std::string, uint32_t> index_of;  // GPU type id -> table index
+    for (uint32_t g = 0; g < (uint32_t)offers_.size(); ++g) index_of.emplace(offers_[g].ID, g);
+    const uint32_t G = (uint32_t)offers_.size(), W = (G + 31) / 32;
+    auto upload = [&](const std::vector<std::vector<std::string>>& group) {
+        std::vector<uint32_t> words((size_t)group.size() * W, 0u);
+        for (size_t s = 0; s < group.size(); ++s)
+            for (const auto& id : group[s]) {
+                auto f = index_of.find(id);
+                if (f != index_of.end()) words[s * W + f->second / 32] |= 1u << (f->second & 31);
+            }
+        set_lists_.clear();
+        if (rpk_offer_sets_upload(ctx_, (uint32_t)group.size(), G, words.empty() ? nullptr : words.data()) != RPK_OK) return false;
+        ++set_uploads_;
+        set_lists_ = group;
+        set_table_ = offer_uploads_;
+        return true;
+    };
+    // reuse the resident sets when they were built on this table and hold every list of the batch
+    std::vector<uint32_t> resident_id(lists.size(), UINT32_MAX);
+    bool reuse = may_reuse && set_table_ == offer_uploads_ && !set_lists_.empty();
+    for (size_t l = 0; reuse && l < lists.size(); ++l) {
+        auto f = std::find(set_lists_.begin(), set_lists_.end(), lists[l]);
+        if (f == set_lists_.end()) reuse = false; else resident_id[l] = (uint32_t)(f - set_lists_.begin());
+    }
+    const size_t n_groups = reuse ? 1 : (lists.size() + RPK_MAX_OFFER_SETS - 1) / RPK_MAX_OFFER_SETS;
+    PodColumnsSoA sub;
+    std::vector<uint16_t> set_id;
+    std::vector<int32_t> best, t5;
+    std::vector<uint32_t> rows;
+    for (size_t grp = 0; grp < n_groups; ++grp) {
+        const size_t l0 = grp * RPK_MAX_OFFER_SETS, l1 = std::min(lists.size(), l0 + RPK_MAX_OFFER_SETS);
+        if (!reuse && !upload(std::vector<std::vector<std::string>>(lists.begin() + (long)l0, lists.begin() + (long)l1))) return false;
+        rows.clear();
+        for (uint32_t i = 0; i < P; ++i)
+            if (row_list[i] == UINT32_MAX ? grp == 0 : (row_list[i] >= l0 && row_list[i] < l1)) rows.push_back(i);
+        const uint32_t n = (uint32_t)rows.size();
+        if (n == 0) continue;
+        sub.resize(n); set_id.resize(n); best.resize(n); t5.resize((size_t)n * RPK_TOPK);
+        for (uint32_t j = 0; j < n; ++j) {
+            const uint32_t i = rows[j];
+            sub.req_mem_gb[j] = cols.req_mem_gb[i]; sub.req_vcpu[j] = cols.req_vcpu[i]; sub.req_ram_gb[j] = cols.req_ram_gb[i];
+            sub.max_price[j] = cols.max_price[i]; sub.cloud[j] = cols.cloud[i];
+            set_id[j] = row_list[i] == UINT32_MAX ? (uint16_t)RPK_SET_ALL
+                                                  : (uint16_t)(reuse ? resident_id[row_list[i]] : row_list[i] - (uint32_t)l0);
+        }
+        if (rpk_select_sets(ctx_, n, sub.req_mem_gb.data(), sub.req_vcpu.data(), sub.req_ram_gb.data(), sub.max_price.data(),
+                            sub.cloud.data(), set_id.data(), best.data(), t5.data()) != RPK_OK) {
+            if (reuse) set_lists_.clear();  // the engine no longer holds them (e.g. its table was replaced)
+            return false;
+        }
+        ++set_select_calls_;
+        for (uint32_t j = 0; j < n; ++j) std::memcpy(top5 + (size_t)rows[j] * RPK_TOPK, t5.data() + (size_t)j * RPK_TOPK, RPK_TOPK * sizeof(int32_t));
+    }
+    return true;
 }
 
 // processPendingPods -- kubelet.go:747-814: every tracked pod that is Pending and has no RunPod id is

@@ -43,6 +43,8 @@ constexpr const char* PortsAnnotation = "runpod.io/ports";
 constexpr const char* MaxPriceAnnotation = "runpod.io/max-price-per-hr";
 constexpr const char* VcpuAnnotation = "runpod.io/required-vcpu";
 constexpr const char* RamAnnotation = "runpod.io/required-ram-gb";
+// comma-separated GPU type ids the pod may run on (parsed like DatacenterAnnotation, runpod_client.go:1354-1362)
+constexpr const char* GpuTypeIdsAnnotation = "runpod.io/gpu-type-ids";
 constexpr double DefaultMaxPrice = 0.5;  // runpod_client.go:48
 
 // PodStatus enum strings (runpod_client.go:55-64)
@@ -129,12 +131,18 @@ bool MessageHasError(const std::string& message);  // strings.Contains(strings.T
 // the same decision from the 16-bit code the sweep kernel emits next to a changed slot (RPK_CODE_*): no string work
 PodStatusView StatusFromCode(uint16_t code, const std::string& status, const std::string& message);
 
+// runpod.io/gpu-type-ids value -> ids: strings.Split(v, ",") then strings.TrimSpace on each element, exactly like the
+// datacenter list (runpod_client.go:1354-1362); "" (annotation absent) -> no restriction (empty vector)
+std::vector<std::string> ParseGpuTypeIds(const std::string& v);
+
 struct PodColumns {  // one row of the P x G grid
     int32_t req_mem_gb;
     int32_t req_vcpu, req_ram_gb;
     double max_price;
     uint8_t cloud;  // RPK_CLOUD_*
     std::string cloud_type;  // "SECURE" | "COMMUNITY"
+    bool restricted = false;               // runpod.io/gpu-type-ids present (pod, else owner Job)
+    std::vector<std::string> gpu_type_ids; // its parsed list
 };
 PodColumns PrepareColumns(const Pod& pod);  // the annotation half of PrepareRunPodParameters (:1255-1281)
 
@@ -143,7 +151,10 @@ struct PodColumnsSoA {
     std::vector<int32_t> req_mem_gb, req_vcpu, req_ram_gb;
     std::vector<double> max_price;
     std::vector<uint8_t> cloud;
-    void resize(size_t n) { req_mem_gb.resize(n); req_vcpu.resize(n); req_ram_gb.resize(n); max_price.resize(n); cloud.resize(n); }
+    std::vector<std::string> gpu_type_ids;  // raw runpod.io/gpu-type-ids value per row, "" = unrestricted
+    void resize(size_t n) {
+        req_mem_gb.resize(n); req_vcpu.resize(n); req_ram_gb.resize(n); max_price.resize(n); cloud.resize(n); gpu_type_ids.assign(n, "");
+    }
     size_t size() const { return req_mem_gb.size(); }
 };
 // Column ingest for a whole batch: PrepareColumns for every pod, rows split contiguously over n_threads host
@@ -187,6 +198,8 @@ public:
     uint64_t SelectCalls() const { return select_calls_; }
     uint64_t StatusCalls() const { return status_calls_; }
     uint64_t OfferUploads() const { return offer_uploads_; }
+    uint64_t SetSelectCalls() const { return set_select_calls_; }  // rpk_select_sets calls (batches with gpu-type-ids)
+    uint64_t SetUploads() const { return set_uploads_; }
     uint64_t HostCompares() const { return host_compares_; }  // sweeps' pods compared on the host (status longer than any slot)
     uint32_t Stride() const { return stride_; }
     void SetClock(double now_s) { now_ = now_s; }
@@ -201,6 +214,9 @@ private:
     static std::string Key(const std::string& ns, const std::string& name) { return ns + "-" + name; }  // kubelet.go:386
     bool RefreshOffersLocked(std::string* err);  // engine_mutex_ held
     bool DeployBatch(const std::vector<std::string>& keys);
+    // restricted rows of a batch: distinct gpu-type-ids lists -> offer sets -> rpk_select_sets (engine_mutex_ held);
+    // may_reuse = false uploads the sets even if they look resident
+    bool SelectWithSetsLocked(const PodColumnsSoA& cols, int32_t* top5, bool may_reuse = true);
     void Notify(const PodPtr& pod);
     uint32_t AllocSlot();
     void SeedSlot(uint32_t slot);                // device previous state of ONE slot := records_[slot]
@@ -226,7 +242,10 @@ private:
     uint32_t max_pods_;
     ProviderOptions opt_;
     double now_ = 0;
-    uint64_t select_calls_ = 0, status_calls_ = 0, offer_uploads_ = 0;
+    uint64_t select_calls_ = 0, status_calls_ = 0, offer_uploads_ = 0, set_select_calls_ = 0, set_uploads_ = 0;
+    // offer sets resident on the engine: set s = the ids of set_lists_[s], built on table upload number set_table_
+    std::vector<std::vector<std::string>> set_lists_;
+    uint64_t set_table_ = 0;
 };
 
 }  // namespace rpkhost

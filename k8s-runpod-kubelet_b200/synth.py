@@ -108,6 +108,40 @@ def make_pods(P: int, seed: int = SEED, reference_exact: bool = False, row0: int
     }
 
 
+SET_ALL = 0xFFFF  # RPK_SET_ALL: an unrestricted row
+# offer-set sizes, cycled over the set index: empty, one offer, 1 %, 10 %, 50 %, every offer
+SET_FRACTIONS = (0.0, None, 0.01, 0.10, 0.50, 1.0)
+
+
+def make_offer_sets(G: int, n_sets: int, seed: int = SEED) -> np.ndarray:
+    """bool ``(n_sets, G)`` membership of ``n_sets`` offer sets (the ``runpod.io/gpu-type-ids`` lists of a batch).
+    Set s has the size class ``SET_FRACTIONS[s % 6]``: empty, a single offer (drawn per set), or each offer
+    independently with that probability (all offers for 1.0)."""
+    rows = np.arange(G, dtype=np.uint64)
+    out = np.zeros((n_sets, G), bool)
+    for s in range(n_sets):
+        f = SET_FRACTIONS[s % len(SET_FRACTIONS)]
+        if f is None:
+            if G:
+                out[s, int(r(300 + s, np.zeros(1, np.uint64), seed)[0] % np.uint64(G))] = True
+        elif f >= 1.0:
+            out[s] = True
+        elif f > 0.0:
+            out[s] = (r(300 + s, rows, seed) % np.uint64(1_000_000)) < np.uint64(int(f * 1_000_000))
+    return out
+
+
+def make_set_ids(P: int, n_sets: int, frac_restricted: float, seed: int = SEED, row0: int = 0) -> np.ndarray:
+    """uint16 set id per pod row [row0, row0+P): a row is restricted with probability ``frac_restricted`` (to a set drawn
+    uniformly), else ``SET_ALL``; 1 % of the restricted rows carry an id >= n_sets (no such set: nothing feasible)."""
+    rows = np.arange(row0, row0 + P, dtype=np.uint64)
+    restricted = (r(50, rows, seed) % np.uint64(1_000_000)) < np.uint64(int(frac_restricted * 1_000_000))
+    ids = (r(51, rows, seed) % np.uint64(max(n_sets, 1))).astype(np.int64)
+    unknown = ((r(52, rows, seed) % np.uint64(100)) < np.uint64(1)) | (n_sets == 0)
+    ids = np.where(unknown, n_sets + (r(53, rows, seed) % np.uint64(7)).astype(np.int64), ids)
+    return np.where(restricted, ids, SET_ALL).astype(np.uint16)
+
+
 def encode_record(status: bytes, ports_exposed: bool, stride: int = 32, msg_error: bool = False) -> np.ndarray:
     """Canonical slot ``[b0][status][0x00][ports][pad]``, b0 = len | flag << 7, len = len(status)+2 <= min(stride-1, 127);
     the flag bit ("statusMessage contains error/fail", kubelet.go:1907) is not a compared field and is not hashed."""

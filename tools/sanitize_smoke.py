@@ -1,5 +1,5 @@
 """Small end-to-end run for compute-sanitizer (memcheck / racecheck / synccheck): every kernel kind, top-5,
-the latency and the pipelined host paths, both status kernels.  Usage on the GPU box:
+the latency and the pipelined host paths, both status kernels, offer sets.  Usage on the GPU box:
     compute-sanitizer --tool memcheck python tools/sanitize_smoke.py
 """
 import os
@@ -12,6 +12,43 @@ import oracle  # noqa: E402
 import rpk  # noqa: E402
 
 ONLY_MULTI = os.environ.get("RPK_SANITIZE_ONLY_MULTI") == "1"  # the 2-GPU part alone (a 2-GPU box is charged twice)
+ONLY_SETS = os.environ.get("RPK_SANITIZE_ONLY_SETS") == "1"    # the offer-set part alone
+
+
+def sets_part():
+    """Offer sets: set build (compact / gather / ingest / remap) with empty, one-offer and full sets, and rpk_select_sets
+    on the host and device entry points (partition, per-set selects, un-permute), top-5 included, against the oracle."""
+    import torch
+
+    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
+    import sets_restatement as sr
+
+    es = rpk.Engine(1)
+    G = 5000
+    so = rpk.synth.make_offers(G, correlated=True, seed=4)
+    members = rpk.synth.make_offer_sets(G, 7, seed=4)
+    es.upload_offers(so)
+    es.upload_offer_sets(members)
+    for P in (37, 20_001):  # fused kernel per bin / persistent kernel for the large bins
+        pods = rpk.synth.make_pods(P, seed=P)
+        ids = rpk.synth.make_set_ids(P, 7, 0.6, seed=P)
+        ob, ot = sr.oracle_select_sets(so, pods, members, ids)
+        b, t = es.select_sets(pods, ids, want_top5=True)
+        assert np.array_equal(b, ob) and np.array_equal(t, ot), ("sets host", P)
+        d = {k: torch.from_numpy(v).cuda() for k, v in pods.items()}
+        d_best = torch.empty(P, dtype=torch.int32, device="cuda")
+        d_top5 = torch.empty(P * 5, dtype=torch.int32, device="cuda")
+        es.select_sets_device(d, torch.from_numpy(ids.view(np.int16)).cuda(), d_best, d_top5)
+        torch.cuda.synchronize()
+        assert np.array_equal(d_best.cpu().numpy(), ob) and np.array_equal(d_top5.cpu().numpy().reshape(P, 5), ot), ("sets device", P)
+    es.close()
+    print("sanitize_smoke offer-set part ok")
+
+
+if ONLY_SETS:
+    sets_part()
+    print("sanitize_smoke ok")
+    sys.exit(0)
 eng = rpk.Engine(1)
 offers = rpk.synth.make_offers(20_000, correlated=True)
 for force in () if ONLY_MULTI else (None, "bitmap_grouped", "bitmap_grid", "packed_pos", "packed", "generic"):
@@ -74,6 +111,9 @@ for P in (20_001, 70_003):
         assert np.array_equal(va[3:].cpu().numpy(), ob) and np.array_equal(vb[3:].cpu().numpy(), ob), P
         assert int((va[:3] != -9).sum()) == 0 and int((vb[:3] != -9).sum()) == 0
 eng.close()
+
+if not ONLY_MULTI:
+    sets_part()
 
 # two GPUs: the fused push + signal + wait, and the sharded sweep's exchange (racecheck / memcheck see peer stores)
 if torch.cuda.device_count() >= 2:
